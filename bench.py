@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed, DIR/<name>.npy
 
 A "step" is one PPO update: rollout of T=128 steps over the local envs, GAE, and
 update_epochs x num_minibatches clipped-surrogate minibatch updates (ppo.jl:117-253).
@@ -59,7 +60,12 @@ def parse():
                          "(crl_dqn_comm_init: envs, replay and batch sharded, one gradient allreduce per learning step)")
     ap.add_argument("--algo", default="ppo", choices=["ppo", "a2c", "dqn"],
                     help="a2c = BASELINE.json configs[2]: A2C CartPole, 16384 envs, n-step returns + fused update (1 GPU)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 L2_NOTE = ("not flushed: every step regenerates its 16.5 MB rollout buffer on the device (L2-resident in production too); "
@@ -147,6 +153,43 @@ def measured_peaks():
         return json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
     except Exception:
         return None
+
+
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_BYTES = 60 << 20   # array data; with the .npy headers the files stay under 64 MB
+# the rollout buffer the last update trained on (env axis 1) and the env vector's next observation (env axis 0)
+PPO_DUMP_FIELDS = (("obs", "CRL_F_STATE", 1), ("action", "CRL_F_ACTION", 1), ("logprob", "CRL_F_LOGPROB", 1),
+                   ("reward", "CRL_F_REWARD", 1), ("terminal", "CRL_F_TERMINAL", 1), ("value", "CRL_F_VALUE", 1),
+                   ("advantage", "CRL_F_ADVANTAGE", 1), ("return", "CRL_F_RETURN", 1), ("next_obs", "CRL_F_NEXT_OBS", 0))
+
+
+def ppo_outputs(h, stats, agg):
+    """what a caller of train_update + fetch_update has after the last update: the parameters, the loss statistics of
+    every minibatch, the episode aggregate and the rollout buffer. Returns (arrays, {name: (array, env axis)})."""
+    from cleanrl_jl_b200 import _abi
+    whole = {"params": h.get_params(), "loss_stats": stats,
+             "episode_agg": np.array([agg.count, agg.sum_return, agg.sum_length, agg.max_return, agg.dropped], np.float64)}
+    per_env = {name: (h.read_field(getattr(_abi, field)), axis) for name, field, axis in PPO_DUMP_FIELDS}
+    return whole, per_env
+
+
+def dump_outputs(out_dir, whole, per_env=None, n_envs=0):
+    """writes every array as out_dir/<name>.npy, in float64 where the library computes it in float64 and float32
+    otherwise. If all of it exceeds DUMP_BYTES, the arrays with an env axis keep a fixed, seeded sample of the envs,
+    whose indices go to env_index.npy."""
+    cast = lambda a: a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+    whole = {k: cast(a) for k, a in whole.items()}
+    per_env = {k: (cast(a), axis) for k, (a, axis) in (per_env or {}).items()}
+    fixed = sum(a.nbytes for a in whole.values())
+    env_bytes = sum(a.nbytes for a, _ in per_env.values())
+    if fixed + env_bytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - fixed - 8 * n_envs) * n_envs // env_bytes
+        idx = np.sort(np.random.default_rng(0).choice(n_envs, keep, replace=False))
+        whole["env_index"] = idx.astype(np.float64)
+        per_env = {k: (np.take(a, idx, axis=axis), axis) for k, (a, axis) in per_env.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in list(whole.items()) + [(k, a) for k, (a, _) in per_env.items()]:
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------ CPU baseline (oracle port)
@@ -351,6 +394,10 @@ def run_dqn(args):
     st = h.run(ITERS)                              # the last call reads the statistics back = stream synchronisation
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        q, target = h.get_params()
+        dump_outputs(args.dump_outputs, {"q_params": q, "target_params": target, "stats": np.array(
+            [st.last_loss, st.sum_return, st.sum_length, st.epsilon, st.episodes, st.learn_steps, st.iterations], np.float64)})
     h.close()
     wall = parallel.max_over_ranks(wall * 1e3) * 1e-3
     value = args.steps * ITERS * N * world / wall
@@ -624,6 +671,8 @@ def run_ours(args):
     launches = h.kernel_launches() - launches0
     value = args.steps * B_local * world / (ms_total * 1e-3)
     stats, agg = h.fetch_update()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *ppo_outputs(h, stats, agg), n_envs=n_local)
 
     # ---- per-kernel device time (CUDA events on the handle's stream, graphs off for this pass)
     h.profile(True)
