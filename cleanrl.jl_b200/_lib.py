@@ -71,6 +71,8 @@ SIGNATURES = {
     "crl_dqn_run": (C.c_int, [V, I64, V]),
     "crl_dqn_comm_init": (C.c_int, [V, V, I32, I32, I32]),
     "crl_dqn_read_buffer": (C.c_int, [V] * 8),
+    "crl_dqn_forward_raw": (C.c_int, [V, V, V, I64, V]),
+    "crl_dqn_loss_raw": (C.c_int, [V, V, I32] + [V] * 5 + [F64, V, V, V]),
     "crl_tb_open": (C.c_int, [C.c_char_p, C.POINTER(V)]),
     "crl_tb_scalars": (C.c_int, [V, F64, I64, I32, C.c_char_p, V]),
     "crl_tb_flush": (C.c_int, [V]),

@@ -22,6 +22,8 @@
 //                         tile of dW2 (or per element of the small arrays) sums over the batch in ascending sample
 //                         order (deterministic, the oracle's order) and applies Adam to the parameters it has just
 //                         differentiated (plus the target copy), so gradients never leave registers.
+// crl_dqn_forward_raw and crl_dqn_loss_raw run the acting kernel's forward pass and the two learning kernels (gradient
+// out instead of Adam) on rows the caller passes in, so that each can be compared with a reference on its own.
 // Every decision that only depends on counters (epsilon, "learn on this iteration?", "copy the target?", Adam's beta
 // powers) is taken on the host, so a run is a plain sequence of launches on one stream without any device-to-host read.
 #include <math.h>
@@ -374,6 +376,29 @@ __global__ void __launch_bounds__(ACT_THREADS, 1) dqn_act_kernel(ActArgs a) {
   }
 }
 
+// crl_dqn_forward_raw: the acting kernel's forward pass alone (same instantiation of q_forward, 32 samples per CTA, named
+// barrier), so that its Q-values can be compared with a reference; rows past n are zero and not written back
+__global__ void __launch_bounds__(ACT_T, 1) dqn_forward_raw_kernel(const float* q, const float* obs, float* q_out, int64_t n) {
+  extern __shared__ __align__(16) float smem[];
+  constexpr int SP = ACT_SP;
+  float* p = smem;                       // [DQ_PP]
+  float* h1 = p + DQ_PP;                 // [120][SP]
+  float* h2 = h1 + DQ_H1 * SP;           // [84][SP]
+  float* qo = h2 + DQ_H2 * SP;           // [2][SP]
+  float* xs = qo + DQ_A * SP;            // [4][SP]
+  const int tid = threadIdx.x;
+  load_q_params<ACT_T>(q, p, tid);
+  const int64_t i = (int64_t)blockIdx.x * ACT_E + tid;
+  if (tid < ACT_E) {
+    float4 x = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    if (i < n) x = reinterpret_cast<const float4*>(obs)[i];
+    xs[0 * SP + tid] = x.x; xs[1 * SP + tid] = x.y; xs[2 * SP + tid] = x.z; xs[3 * SP + tid] = x.w;
+  }
+  __syncthreads();
+  q_forward<ACT_E, SP, ACT_T, 1>(p, xs, h1, h2, qo, tid);
+  if (tid < ACT_E && i < n) reinterpret_cast<float2*>(q_out)[i] = make_float2(qo[0 * SP + tid], qo[1 * SP + tid]);
+}
+
 struct LearnArgs {
   float* q; float* tgt; float* m; float* v;
   const float *b_state, *b_next, *b_reward; const int* b_action; const uint8_t* b_term;
@@ -381,6 +406,7 @@ struct LearnArgs {
   unsigned long long seed, learn_step;
   double gamma, lr;
   int B, size, copy_target;
+  int in_order;           // sample b is row b of the b_* arrays (crl_dqn_loss_raw), not entry b of the keyed permutation
   // sample-major scratch between the two kernels: [128][120], [128][84], [128][84], [128][120], [128][4], [128][2]
   float *h1T, *h2T, *z2T, *z1T, *xT, *dqT;
   double* loss_part;      // [LF_MAX_BLOCKS]
@@ -436,10 +462,13 @@ __global__ void __launch_bounds__(LF_T) dqn_learn_fwd_kernel(LearnArgs a) {
   float rew = 0.0f;
   if (tid < LF_S && b0 + tid < B) {
     // sample(1:size, B, replace=false), replay_buffer.jl:43: the first B entries of a keyed permutation of [0,size)
-    uint32_t keys[8];
-    philox_draw(a.seed, (uint32_t)a.rank, a.learn_step, STREAM_DQN_BATCH, keys);
-    philox_draw(a.seed, 0x80000000u | (uint32_t)a.rank, a.learn_step, STREAM_DQN_BATCH, keys + 4);
-    const uint32_t idx = perm_index((uint32_t)(b0 + tid), (uint32_t)a.size, perm_half_bits((uint32_t)a.size), keys);
+    uint32_t idx = (uint32_t)(b0 + tid);
+    if (!a.in_order) {
+      uint32_t keys[8];
+      philox_draw(a.seed, (uint32_t)a.rank, a.learn_step, STREAM_DQN_BATCH, keys);
+      philox_draw(a.seed, 0x80000000u | (uint32_t)a.rank, a.learn_step, STREAM_DQN_BATCH, keys + 4);
+      idx = perm_index(idx, (uint32_t)a.size, perm_half_bits((uint32_t)a.size), keys);
+    }
     s4 = reinterpret_cast<const float4*>(a.b_state)[idx];
     n4 = reinterpret_cast<const float4*>(a.b_next)[idx];
     act = a.b_action[idx];
@@ -782,8 +811,11 @@ __global__ void __launch_bounds__(256) dqn_adam_kernel(LearnArgs a) {
   dqn_adam<1>(a, idx, g, ok);
 }
 
+__global__ void dqn_loss_raw_finish_kernel(const double* sq, int B, double* loss_out) { *loss_out = sq[0] / (double)B; }
+
 constexpr int ACT_SPEC_FLOATS = (4 + 2 * 4 + 4 + 2 + 1 + 1) * ACT_E;   // state | 2 successors | reset state | uniform (double) | random bit | used flag
-constexpr size_t ACT_SMEM = (DQ_PP + (DQ_H1 + DQ_H2 + DQ_A + DQ_D) * ACT_SP + ACT_SPEC_FLOATS) * sizeof(float);
+constexpr size_t FWD_RAW_SMEM = (DQ_PP + (DQ_H1 + DQ_H2 + DQ_A + DQ_D) * ACT_SP) * sizeof(float);
+constexpr size_t ACT_SMEM = FWD_RAW_SMEM + ACT_SPEC_FLOATS * sizeof(float);
 constexpr size_t LF_SMEM = (2 * DQ_PP + (DQ_H1 + DQ_H2 + 2 * DQ_A + 2 * DQ_D) * LF_SP) * sizeof(float);
 constexpr size_t LU_SMEM = ((size_t)LEARN_B * (DQ_H2 + LU_KA) + DQ_H2 * LU_KA) * sizeof(float);   // kind (A) is the largest
 static_assert(LEARN_B * (LU_JB + DQ_D) <= LEARN_B * (DQ_H2 + LU_KA) && LEARN_B * (2 * LU_KC + DQ_A) <= LEARN_B * (DQ_H2 + LU_KA), "upd smem");
@@ -1118,5 +1150,76 @@ extern "C" CRL_API int crl_dqn_read_buffer(crl_dqn_ctx* c, float* state, int32_t
   DCK(cudaStreamSynchronize(c->stream));
   if (size) *size = c->size;
   if (ptr) *ptr = c->ptr;
+  return CRL_OK;
+}
+
+static int dqn_raw_device_check() {
+  int dev = 0;
+  DCK(cudaGetDevice(&dev));
+  cudaDeviceProp prop;
+  DCK(cudaGetDeviceProperties(&prop, dev));
+  if (prop.major != 10) return dfail(CRL_ERR_CUDA, "libcleanrl_cuda is built for sm_100a only");
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_dqn_forward_raw(const float* params, const float* obs, float* q_out, int64_t n, void* stream) {
+  if (n < 0 || (n > 0 && (!params || !obs || !q_out))) return dfail(CRL_ERR_INVALID, "NULL argument or n < 0");
+  if (((uintptr_t)params | (uintptr_t)obs) % 16 || (uintptr_t)q_out % 8)
+    return dfail(CRL_ERR_INVALID, "params and obs must be 16-byte aligned, q_out 8-byte aligned");
+  if (n == 0) return CRL_OK;
+  if (int rc = dqn_raw_device_check()) return rc;
+  DCK(cudaFuncSetAttribute(dqn_forward_raw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FWD_RAW_SMEM));
+  const int64_t grid = (n + ACT_E - 1) / ACT_E;
+  if (grid > 0x7fffffff) return dfail(CRL_ERR_INVALID, "n too large");
+  dqn_forward_raw_kernel<<<(unsigned)grid, ACT_T, FWD_RAW_SMEM, (cudaStream_t)stream>>>(params, obs, q_out, n);
+  DCK(cudaGetLastError());
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_dqn_loss_raw(const float* q, const float* tgt, int32_t B, const float* state, const int32_t* action,
+                                        const float* reward, const float* next_state, const uint8_t* terminal, double gamma,
+                                        float* grads_out, double* loss_out, void* stream) {
+  if (!q || !tgt || !state || !action || !reward || !next_state || !terminal || !grads_out || !loss_out)
+    return dfail(CRL_ERR_INVALID, "NULL argument");
+  if (B < 1 || B > LEARN_B) return dfail(CRL_ERR_INVALID, "B must be in [1, 128]");
+  if (((uintptr_t)q | (uintptr_t)tgt | (uintptr_t)state | (uintptr_t)next_state) % 16)
+    return dfail(CRL_ERR_INVALID, "q, tgt, state and next_state must be 16-byte aligned");
+  if (int rc = dqn_raw_device_check()) return rc;
+  DCK(cudaFuncSetAttribute(dqn_learn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LF_SMEM));
+  DCK(cudaFuncSetAttribute(dqn_learn_upd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LU_SMEM));
+  const cudaStream_t s = (cudaStream_t)stream;
+  // the learning step of crl_dqn_run on rows 0..B-1, its update kernel in the variant that leaves the gradient in gbuf
+  // (= grads_out) and the squared-error sum in lbuf instead of applying Adam (no peers: x_push does nothing)
+  LearnArgs l;
+  memset(&l, 0, sizeof(l));
+  l.q = const_cast<float*>(q); l.tgt = const_cast<float*>(tgt);
+  l.b_state = state; l.b_next = next_state; l.b_reward = reward; l.b_action = action; l.b_term = terminal;
+  l.gamma = gamma; l.B = B; l.size = B; l.in_order = 1; l.B_scale = B; l.gbuf = grads_out;
+  float* scratch = nullptr;
+  double* dscratch = nullptr;
+  const size_t nf = (size_t)LEARN_B * (2 * DQ_H1 + 2 * DQ_H2 + DQ_D + DQ_A);
+  DCK(cudaMalloc(reinterpret_cast<void**>(&scratch), nf * sizeof(float)));
+  if (cudaMalloc(reinterpret_cast<void**>(&dscratch), (LF_MAX_BLOCKS + 1) * sizeof(double)) != cudaSuccess) {
+    cudaFree(scratch);
+    return dfail(CRL_ERR_CUDA, "cudaMalloc failed (crl_dqn_loss_raw)");
+  }
+  l.h1T = scratch; l.z1T = l.h1T + LEARN_B * DQ_H1; l.h2T = l.z1T + LEARN_B * DQ_H1; l.z2T = l.h2T + LEARN_B * DQ_H2;
+  l.xT = l.z2T + LEARN_B * DQ_H2; l.dqT = l.xT + LEARN_B * DQ_D;
+  l.loss_part = dscratch; l.lbuf = dscratch + LF_MAX_BLOCKS;
+  const int fwd_blocks = (B + LF_S - 1) / LF_S;
+  dqn_learn_fwd_kernel<<<fwd_blocks, LF_T, LF_SMEM, s>>>(l);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) {
+    dqn_learn_upd_kernel<true><<<LU_A_BLOCKS + LU_B_BLOCKS + LU_C_BLOCKS, LU_T, LU_SMEM, s>>>(l, fwd_blocks);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) {
+    dqn_loss_raw_finish_kernel<<<1, 1, 0, s>>>(l.lbuf, B, loss_out);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);   // the scratch is freed below
+  cudaFree(scratch);
+  cudaFree(dscratch);
+  if (e != cudaSuccess) return dfail(CRL_ERR_CUDA, std::string("crl_dqn_loss_raw failed: ") + cudaGetErrorString(e));
   return CRL_OK;
 }

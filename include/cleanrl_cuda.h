@@ -334,6 +334,17 @@ CRL_API int crl_dqn_comm_init(crl_dqn_ctx* ctx, const void* id128, int32_t world
  * reward float, terminal uint8; size/ptr as in replay_buffer.jl:11-12 (ptr 0-based) */
 CRL_API int crl_dqn_read_buffer(crl_dqn_ctx* ctx, float* state, int32_t* action, float* reward, float* next_state,
                         uint8_t* terminal, int32_t* size, int32_t* ptr);
+/* Raw DQN kernels (DEVICE pointers; stream = cudaStream_t or NULL), the ones crl_dqn_run launches:
+ * crl_dqn_forward_raw: q_net(obs) (dqn.jl:56) by the acting kernel's forward pass. params float [10934] and
+ * obs float [n][4] 16-byte aligned, q_out float [n][2] 8-byte aligned.
+ * crl_dqn_loss_raw: loss and gradient of one batch (dqn.jl:96-108) by the learning step's two kernels, with sample b
+ * taken from row b of state / action / reward / next_state / terminal (nothing sampled; rows >= B are not read).
+ * q, tgt float [10934]; 1 <= B <= 128; grads_out float [10934] (the un-stepped gradient of Flux.mse, flat order);
+ * loss_out 1 double = mean squared TD error. Allocates and frees its scratch: synchronises `stream`. */
+CRL_API int crl_dqn_forward_raw(const float* params, const float* obs, float* q_out, int64_t n, void* stream);
+CRL_API int crl_dqn_loss_raw(const float* q, const float* tgt, int32_t B, const float* state, const int32_t* action,
+                     const float* reward, const float* next_state, const uint8_t* terminal, double gamma,
+                     float* grads_out, double* loss_out, void* stream);
 
 /* ---- logger hook: TensorBoard event files (logger.jl:7-29, TBLogger; records of ppo.jl:157,247) -------------------
  * Native writer for the "<message>/<key>" scalars the @info records become in TensorBoardLogger.jl. One call = one

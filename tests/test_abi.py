@@ -17,11 +17,13 @@ def header_symbols():
     return sorted(set(re.findall(r"CRL_API\s+(?:int|const char\*)\s+(crl_\w+)\s*\(", src)))
 
 
-def test_header_declares_the_expected_surface():
+def test_header_declares_the_expected_surface_with_the_dqn_raw_kernels():
+    """the 50 entry points before the raw DQN kernels plus crl_dqn_forward_raw and crl_dqn_loss_raw"""
     syms = header_symbols()
-    assert len(syms) == 50
+    assert len(syms) == 52
     for s in ("crl_create", "crl_rollout", "crl_gae", "crl_update_minibatch", "crl_train_update", "crl_gae_raw",
-              "crl_env_step_raw", "crl_policy_forward_raw", "crl_ppo_loss_raw", "crl_clip_adam_raw", "crl_comm_init", "crl_dqn_run", "crl_dqn_comm_init"):
+              "crl_env_step_raw", "crl_policy_forward_raw", "crl_ppo_loss_raw", "crl_clip_adam_raw", "crl_comm_init", "crl_dqn_run",
+              "crl_dqn_comm_init", "crl_dqn_forward_raw", "crl_dqn_loss_raw"):
         assert s in syms
 
 

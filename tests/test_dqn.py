@@ -47,6 +47,73 @@ def _rand_batch(rng, B):
     return s, a, r, s2, term
 
 
+# flat parameter arrays of the Q-network (Flux.params order) and the per-array gradient tolerance of the suite
+DQN_ARRAYS = (("W1", 0, 480), ("b1", 480, 600), ("W2", 600, 10680), ("b2", 10680, 10764), ("W3", 10764, 10932), ("b3", 10932, 10934))
+
+
+def assert_grad_close(g, ref, rtol=1e-4, atol_frac=2e-6, what=""):
+    """per parameter array: |g - ref| <= rtol |ref| + atol_frac * max|ref of that array|"""
+    for name, a, b in DQN_ARRAYS:
+        np.testing.assert_allclose(g[a:b], ref[a:b], rtol=rtol, atol=atol_frac * np.abs(ref[a:b]).max(), err_msg=what + name)
+
+
+def edge_batch(kind, B, seed):
+    """(q, tgt, state, action, reward, next_state, terminal, gamma) of one of the edge batches the DQN loss is tested at.
+    tgt != q everywhere; rewards are -1.5, 1 or 2 so that no TD error is close to 0 (a float32 Q-value then decides the
+    relative error of the whole gradient, which would make the per-array tolerance depend on luck rather than on the
+    kernel). Kinds:
+      mixed     random actions, 20 % terminal, gamma 0.99
+      action0   every action 0: column 1 of dq is 0, so dW3 row 1 and db3[1] are exactly 0
+      terminal  every sample terminal (the target net drops out), gamma 0.99
+      open      no sample terminal, gamma 1
+      gamma0    no sample terminal, gamma 0
+      relu0     every state row 0, every other b1 entry 0 and the second-layer units 0, 7, 14, ... with zero weights and
+                bias: those first- and second-layer pre-activations are exactly 0, and relu'(0) = 0 (Flux) makes their
+                gradients exactly 0"""
+    from cleanrl_jl_b200.dqn_algo import init_q_params
+    rng = np.random.default_rng(seed)
+    q = init_q_params(seed)
+    q[480:600] = rng.normal(0, 0.2, 120)
+    q[10680:10764] = rng.normal(0, 0.1, 84)
+    q[10932:] = rng.normal(0, 0.1, 2)
+    tgt = init_q_params(seed + 1000)
+    tgt[480:600] = rng.normal(0, 0.2, 120)
+    s = rng.uniform(-2, 2, (B, 4)).astype(F)
+    s2 = rng.uniform(-2, 2, (B, 4)).astype(F)
+    a = rng.integers(0, 2, B).astype(np.int32)
+    r = rng.choice(np.array([-1.5, 1.0, 2.0], F), B)
+    term = (rng.random(B) < 0.2).astype(np.uint8)
+    gamma = 0.99
+    if kind == "action0":
+        a[:] = 0
+    elif kind == "terminal":
+        term[:] = 1
+    elif kind == "open":
+        term[:] = 0
+        gamma = 1.0
+    elif kind == "gamma0":
+        term[:] = 0
+        gamma = 0.0
+    elif kind == "relu0":
+        s[:] = 0.0
+        q[480:600:2] = 0.0
+        q[600:10680].reshape(120, 84)[:, ::7] = 0.0      # W2 (84 x 120) column-major: rows 0, 7, ... of W2
+        q[10680:10764:7] = 0.0
+    else:
+        assert kind == "mixed", kind
+    return q, tgt, s, a, r, s2, term, gamma
+
+
+def relu0_zero_indices():
+    """gradient entries that must be exactly 0 in the relu0 batch: all of dW1 (the states are 0), db1 of the zero-bias
+    first-layer units, and dW2 row / db2 / dW3 column of the dead second-layer units"""
+    w2 = np.zeros((84, 120), bool)
+    w2[::7, :] = True
+    dead = np.arange(0, 84, 7)
+    return np.concatenate([np.arange(0, 480), 480 + np.arange(0, 120, 2), 600 + np.flatnonzero(w2.ravel(order="F")),
+                           10680 + dead, 10764 + 2 * dead, 10764 + 2 * dead + 1])
+
+
 def test_oracle_linear_schedule_matches_dqn_jl(olib, abi):
     o = OracleDQN(olib, abi.make_dqn_config())
     # dqn.jl:28-31 with the defaults 1.0 -> 0.05 over 10,000 steps
@@ -72,8 +139,31 @@ def test_oracle_forward_and_gradient_match_float64_numpy(olib, abi):
     np.testing.assert_allclose(qo, qn, rtol=2e-5, atol=2e-6)
     g, loss = o.loss_raw(q, tgt, s, a, r, s2, term, 0.99)
     gn, lossn = _np_loss_grad(q, tgt, s, a, r, s2, term, 0.99)
-    assert abs(loss - lossn) < 1e-5 * abs(lossn)
-    np.testing.assert_allclose(g, gn, rtol=1e-3, atol=2e-6 * np.abs(gn).max())
+    # achieved here: loss 1e-8 relative; per array at most 3.5e-7 of the array's max|g| away, 0.11 of the bound below
+    assert abs(loss - lossn) < 1e-7 * abs(lossn)
+    assert_grad_close(g, gn, rtol=1e-5, atol_frac=1e-6)
+    o.close()
+
+
+@pytest.mark.parametrize("kind", ["mixed", "action0", "terminal", "open", "gamma0", "relu0"])
+@pytest.mark.parametrize("B", [1, 2, 16, 17, 33, 100, 128])
+def test_oracle_dqn_loss_at_the_edges_matches_float64_numpy(olib, abi, kind, B):
+    """the reference the GPU loss kernels are compared with, pinned at the same edge batches: per array rtol 1e-4, atol
+    2e-6 max|g| (achieved: at most 0.07 of that bound at every batch size of the GPU tests), loss rtol 1e-6 (achieved:
+    5.4e-7), and the entries that must be exactly 0 are exactly 0"""
+    o = OracleDQN(olib, abi.make_dqn_config())
+    q, tgt, s, a, r, s2, term, gamma = edge_batch(kind, B, seed=B)
+    g, loss = o.loss_raw(q, tgt, s, a, r, s2, term, gamma)
+    gn, lossn = _np_loss_grad(q, tgt, s, a, r, s2, term, gamma)
+    assert abs(loss - lossn) <= 1e-6 * lossn
+    assert_grad_close(g, gn)
+    if kind == "action0":
+        assert np.all(g[10765:10932:2] == 0) and g[10933] == 0 and np.all(gn[10765:10932:2] == 0)
+        assert np.abs(g[10764:10932:2]).max() > 0 and g[10932] != 0
+    if kind == "relu0":
+        z = relu0_zero_indices()
+        assert np.all(g[z] == 0) and np.all(gn[z] == 0)
+        assert np.count_nonzero(g[480:600]) >= 20 and np.count_nonzero(g[10680:10764]) >= 20   # the live units learn
     o.close()
 
 
