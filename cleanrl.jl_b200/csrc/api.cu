@@ -685,9 +685,9 @@ static int enqueue_minibatch(crl_ctx* c, const IdxSrc& ix, int M, double lr_host
   ua.tc_net_a = c->L.critic - c->L.actor; ua.tc_net_c = (c->L.continuous ? c->L.logstd : c->L.P) - c->L.critic;
   ua.values_fresh = spec ? 1 : 0;       // throughput path: the rollout that filled `value` used the current parameters
   // Fused tail: the tcgen05 kernel reduces, exchanges and applies clip + Adam itself (one cooperative launch per
-  // minibatch). Needs the peer-memory exchange when there are several ranks; CRL_NO_FUSED_TAIL=1 keeps the 3-kernel chain.
-  static const bool fuse_off = getenv("CRL_NO_FUSED_TAIL") != nullptr;
-  const bool want_fuse = (spec || ua.algo == 1) && !fuse_off && (!multi || c->p2p_on);
+  // minibatch). Needs the peer-memory exchange when there are several ranks; the FFMA kernel (CRL_NO_TC=1) and the
+  // NCCL fallback keep the 3-kernel chain.
+  const bool want_fuse = (spec || ua.algo == 1) && (!multi || c->p2p_on);
   loss_grad_tc_plan(&ua, c->sm_count, want_fuse);  // tensor-core kernel when it applies: sets grid_loss / tc_actor_ctas
   AdamArgs aa = adam_args(c, M, lr_host, stats_slot);
   if (spec || ua.algo == 1) {  // the A2C losses have no minibatch-global scalars: the 3-kernel chain is already exact

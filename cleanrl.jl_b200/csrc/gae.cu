@@ -10,8 +10,6 @@
 // The recurrence runs in Float64 exactly as the reference's promotion rules dictate
 // (nonterm = 1.0 .- terminals and gae = 0.0 are Float64, ppo.jl:63,65) and uses _rn intrinsics
 // so that no mul+add is contracted: results are bit-identical to the oracle.
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "kernels.h"
@@ -187,15 +185,10 @@ cudaError_t launch_mode(const float* values, const float* rewards, const uint8_t
   // vectorise only when there are enough threads to fill the machine several times over
   if (vec_ok && N / 4 >= 148LL * 128) {
     const long long nv = N / 4;
-    static int variant = -1;  // tuning hook: CRL_GAE_VARIANT selects the prefetch depth of the vectorised kernel
-    if (variant < 0) { const char* e = getenv("CRL_GAE_VARIANT"); variant = e ? atoi(e) : 0; }
     const unsigned grid = (unsigned)((nv + 127) / 128);
-    // measured on B200 at T=128, N=2^20 (profiles/r1_gae_sweep.txt): U=2 5.9 TB/s, U=4 6.1 TB/s, U=8 4.8 TB/s,
-    // U=16 3.2 TB/s -- deeper prefetch costs occupancy and opens too many DRAM rows at once; U=4 is the default
-    if (variant == 1) gae_kernel<MODE, 4, 8><<<grid, 128, 0, s>>>(values, rewards, dones, next_value, next_done, adv, ret, T, N, gamma, gl);
-    else if (variant == 2) gae_kernel<MODE, 4, 16><<<grid, 128, 0, s>>>(values, rewards, dones, next_value, next_done, adv, ret, T, N, gamma, gl);
-    else if (variant == 3) gae_kernel<MODE, 4, 2><<<grid, 128, 0, s>>>(values, rewards, dones, next_value, next_done, adv, ret, T, N, gamma, gl);
-    else gae_kernel<MODE, 4, 4><<<grid, 128, 0, s>>>(values, rewards, dones, next_value, next_done, adv, ret, T, N, gamma, gl);
+    // prefetch depth U=4: measured on B200 at T=128, N=2^20 (profiles/r1_gae_sweep.txt): U=2 5.9 TB/s, U=4 6.1 TB/s,
+    // U=8 4.8 TB/s, U=16 3.2 TB/s -- deeper prefetch costs occupancy and opens too many DRAM rows at once
+    gae_kernel<MODE, 4, 4><<<grid, 128, 0, s>>>(values, rewards, dones, next_value, next_done, adv, ret, T, N, gamma, gl);
   } else {
     gae_kernel<MODE, 1, 16><<<(unsigned)((N + 127) / 128), 128, 0, s>>>(values, rewards, dones, next_value, next_done,
                                                                        adv, ret, T, N, gamma, gl);

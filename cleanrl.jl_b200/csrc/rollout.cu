@@ -75,9 +75,7 @@ template <int ENV> __device__ __forceinline__ void load_head_row(const float* sp
 
 // both nets forward for the 32 samples whose observations sit in xs; heads -> so[o][e]
 // (o < A: actor logits/mean, o == A: critic value). Called by the 256 forward threads only (named barrier BAR_FWD).
-// HEADREG = false: the output layer reads its weights from shared memory (64 registers fewer: two CTAs per SM when the
-// grid is larger than the GPU)
-template <int ENV, bool HEADREG = true, bool BOOKSYNC = false>
+template <int ENV, bool BOOKSYNC = false>
 __device__ __forceinline__ void forward32(const ThreadCoord<TileGeom<4, 2>>& tc, float* smem, const HeadRow<ENV>& hr,
                                           long long* tr = nullptr) {
   using G = TileGeom<4, 2>;
@@ -108,21 +106,9 @@ __device__ __forceinline__ void forward32(const ThreadCoord<TileGeom<4, 2>>& tc,
     for (int k = 0; k < CRL_H; k++) hv[k] = hrow[k * SP];   // all 64 loads in flight before the (serial) chain starts
     if (BOOKSYNC) nbar_sync(BAR_BOOK, RE * (E::A + 1) + 32);   // the bookkeeping warp has read the previous step's outputs
     float acc = 0.0f;
-    if (HEADREG) {
 #pragma unroll
-      for (int k = 0; k < CRL_H; k++) acc = fmaf(hr.w[k], hv[k], acc);
-      acc += hr.b;
-    } else if (o < E::A) {
-      const float* a = sp + SmemParams<ENV>::ACTOR;
-#pragma unroll
-      for (int k = 0; k < CRL_H; k++) acc = fmaf(a[NetOff<E::D, E::A>::W3 + k * E::A + o], hv[k], acc);
-      acc += a[NetOff<E::D, E::A>::B3 + o];
-    } else {
-      const float* c = sp + SmemParams<ENV>::CRITIC;
-#pragma unroll
-      for (int k = 0; k < CRL_H; k++) acc = fmaf(c[NetOff<E::D, 1>::W3 + k], hv[k], acc);
-      acc += c[NetOff<E::D, 1>::B3];
-    }
+    for (int k = 0; k < CRL_H; k++) acc = fmaf(hr.w[k], hv[k], acc);
+    acc += hr.b;
     so[o * RE + e] = acc;
   }
   RTR(5);
@@ -203,7 +189,7 @@ __device__ __forceinline__ void fwd_layer_8x4(const FwdCoord8x4& fc, const float
   }
 }
 // forward32 for the BIG variant (output layer weights from shared memory)
-template <int ENV, bool BOOKSYNC = false>
+template <int ENV>
 __device__ __forceinline__ void forward32_big(const FwdCoord8x4& fc, float* smem) {
   using E = EnvTraits<ENV>;
   using SM = RolloutSmem<ENV>;
@@ -223,7 +209,7 @@ __device__ __forceinline__ void forward32_big(const FwdCoord8x4& fc, float* smem
   if (threadIdx.x < RE * (E::A + 1)) {
     const int o = threadIdx.x / RE, e = threadIdx.x % RE;
     const float* hrow = h2 + (o < E::A ? 0 : CRL_H) * SP + e;
-    if (BOOKSYNC) nbar_sync(BAR_BOOK, RE * (E::A + 1) + 32);
+    nbar_sync(BAR_BOOK, RE * (E::A + 1) + 32);   // the bookkeeping warp has read the previous step's outputs
     float acc = 0.0f;
     if (o < E::A) {
       const float* a = sp + SmemParams<ENV>::ACTOR;
@@ -457,7 +443,7 @@ __global__ void __launch_bounds__(BIG ? BIG_THREADS : ROLL_THREADS, BIG ? 2 : 1)
       nbar_arrive(BAR_SPEC, RE + 64);
     } else {
       // ends with a barrier of the forward threads; so[] is ready
-      if (BIG) forward32_big<ENV, true>(fc, smem); else forward32<ENV, true, true>(tc, smem, hr);
+      if (BIG) forward32_big<ENV>(fc, smem); else forward32<ENV, true>(tc, smem, hr);
       if (owner) {
         const long long b = (long long)t * a.N + n;
         int act_i = 0;
@@ -585,7 +571,7 @@ __global__ void __launch_bounds__(BIG ? BIG_THREADS : ROLL_THREADS, BIG ? 2 : 1)
     for (int k = 0; k < D; k++) xs[k * SP + e] = fresh[k];
   }
   nbar_sync(BAR_FWD, FWD);
-  if (BIG) forward32_big<ENV, true>(fc, smem); else forward32<ENV, true, true>(tc, smem, hr);
+  if (BIG) forward32_big<ENV>(fc, smem); else forward32<ENV, true>(tc, smem, hr);
   if (valid) {
     a.next_value[n] = so[A * RE + e];
 #pragma unroll

@@ -50,14 +50,10 @@ using namespace crl_upd;
 #endif
 
 constexpr int TC_S = 128;        // samples per tile = TMEM lanes
-#ifndef TC_NG
-#define TC_NG 2                  // feature groups per sample: 2 (8 warps, 32 features per thread); 4 (16 warps, 16 features,
-                                 // 128 registers) measured 7 % slower on B200 and is not validated
-#endif
+constexpr int TC_NG = 2;         // feature groups per sample (8 warps, 32 features per thread)
 constexpr int TC_THREADS = 128 * TC_NG;  // 4 lane quadrants x TC_NG feature groups
 constexpr int TC_WARPS = TC_THREADS / 32;
 constexpr int TC_FG = CRL_H / TC_NG;     // features per thread
-static_assert(TC_NG == 2 || TC_NG == 4, "feature groups per sample");
 constexpr int F_LBO = 144, F_SBO = 32 * F_LBO;  // bytes; feature-major operand: rows r, K = 128 samples
 __device__ __forceinline__ int f_off(int r, int s) { return (r & 7) * 4 + (r >> 3) * (F_SBO / 4) + (s >> 2) * (F_LBO / 4) + (s & 3); }
 // x~^T (rows x_0..x_D-1, ones, zeros): two more 8-row groups (hi, lo) right behind h1^T, same strides, so that
@@ -68,11 +64,8 @@ constexpr int XT_GROUP = F_SBO / 4;  // floats per 8-row group
 // TMEM columns (fp32): z2/dh1 accumulator (A W_hi^T | A_hi W_lo^T: 128) | A operand hi (64) | A operand lo (64) |
 // dW2 accumulator (x h1_hi | x h1_lo | x x~: 144) | dW1,db1 accumulator (x x~_hi | x x~_lo: 16)
 constexpr uint32_t COL_D = 0, COL_AH = 128, COL_AL = 192, COL_D2 = 256, COL_D4 = 400, COL_P = 416, TMEM_COLS = 512;
-// TC_PARK: h1^2 - 1 (the tanh derivative E3 needs) waits in 64 spare TMEM columns from the start of the tile instead of
+// COL_P: h1^2 - 1 (the tanh derivative E3 needs) waits in 64 spare TMEM columns from the start of the tile instead of
 // being rebuilt from the hi/lo rows of h1^T in shared memory (4 scalar loads + an add per feature pair)
-#ifndef TC_PARK
-#define TC_PARK 1
-#endif
 // named barriers: 1-3 hand an operand set to the issuing warp (it syncs, the other warps only arrive), 4-7 = head exchange
 // of lane quadrant 0-3
 constexpr int BAR_G1 = 1, BAR_G3 = 2, BAR_G4 = 3, BAR_X = 4;
@@ -196,11 +189,7 @@ template <int N> __device__ __forceinline__ void tmem_st_n(uint32_t taddr, const
 // compares + 2 selects + 2 sign copies) and (b) the reciprocal is MUFU.RCP without the Newton step (<= 1 ulp). Both are
 // below the 3xTF32 error of the contractions around it (1.2e-6); the rollout and the FFMA kernel keep the exact form.
 // A tanh_fast2 call costs ~35 issue cycles per warp (tools/pipe_probe.cu), 32 calls per thread and tile.
-#ifndef TC_TANH_EXACT
-#define TC_TANH_EXACT 0
-#endif
 __device__ __forceinline__ float2 tanh_upd2(float2 x) {
-  if (TC_TANH_EXACT) return tanh_fast2(x);
   const float lim = 8.1240384f;   // sqrt(66)
   x.x = fminf(fmaxf(x.x, -lim), lim);
   x.y = fminf(fmaxf(x.y, -lim), lim);
@@ -448,11 +437,7 @@ __device__ __forceinline__ void tc_body(const UpdateArgs& a, float* smem, TcBars
   };
 
   // the next tile's first layer is spread over the shadows of G1, G3/G2 and G4 (pairs [0,A), [A,B), [B,end))
-#if defined(TC_L1A) && defined(TC_L1B)
-  constexpr int L1_A = TC_L1A, L1_B = TC_L1B;   // A/B builds
-#else
   constexpr int L1_A = TC_FG / 2 * 3 / 8, L1_B = TC_FG / 2 * 3 / 4;
-#endif
   int it = 0;
   {
     Sample<ENV> cur, nxt;
@@ -491,7 +476,7 @@ __device__ __forceinline__ void tc_body(const UpdateArgs& a, float* smem, TcBars
       TR(2);
       handover(BAR_G1, issue_g1);
       TR(3);
-      if (TC_PARK) {   // not an operand of G1: stored in its shadow (the previous tile's E3 has read its copy: program order)
+      {   // h1^2 - 1 is not an operand of G1: parked in its shadow (the previous tile's E3 has read its copy: program order)
         float dt[TC_FG];
 #pragma unroll
         for (int i = 0; i < TC_FG / 2; i++) {
@@ -687,27 +672,16 @@ __device__ __forceinline__ void tc_body(const UpdateArgs& a, float* smem, TcBars
       if (more) layer1(nxt, h1, IC<L1_A>(), IC<L1_B>());
       TR(10);
 
-      // ---- E3: dz1 = (-dh1) .* (h1^2 - 1), in place over h1^T (whose hi + lo is this tile's h1 exactly)
+      // ---- E3: dz1 = (-dh1) .* (h1^2 - 1), in place over h1^T; h1^2 - 1 comes from the parked TMEM columns
       mbar_wait(bar3, ph);
       TR(11);
       tc_fence_after();
-      float ndh1[TC_FG], ndh1b[TC_FG];
+      float ndh1[TC_FG], ndh1b[TC_FG], dt[TC_FG];
       float2 dz1[TC_FG / 2];
-      if (TC_PARK) {
-        float dt[TC_FG];
-        tmem_ld_triple<TC_FG>(lane_addr + COL_D + f0, lane_addr + COL_D + CRL_H + f0, lane_addr + COL_P + f0, ndh1, ndh1b, dt);
+      tmem_ld_triple<TC_FG>(lane_addr + COL_D + f0, lane_addr + COL_D + CRL_H + f0, lane_addr + COL_P + f0, ndh1, ndh1b, dt);
 #pragma unroll
-        for (int i = 0; i < TC_FG / 2; i++)
-          dz1[i] = __fmul2_rn(__fadd2_rn(f2(ndh1[2 * i], ndh1[2 * i + 1]), f2(ndh1b[2 * i], ndh1b[2 * i + 1])), f2(dt[2 * i], dt[2 * i + 1]));
-      } else {
-        tmem_ld_pair<TC_FG>(lane_addr + COL_D + f0, lane_addr + COL_D + CRL_H + f0, ndh1, ndh1b);
-#pragma unroll
-        for (int i = 0; i < TC_FG / 2; i++) {
-          const float2 h = __fadd2_rn(f2(fh[f_off(f0 + 2 * i, s)], fh[f_off(f0 + 2 * i + 1, s)]),
-                                      f2(fh[f_off(CRL_H + f0 + 2 * i, s)], fh[f_off(CRL_H + f0 + 2 * i + 1, s)]));
-          dz1[i] = __fmul2_rn(__fadd2_rn(f2(ndh1[2 * i], ndh1[2 * i + 1]), f2(ndh1b[2 * i], ndh1b[2 * i + 1])), __ffma2_rn(h, h, f2s(-1.0f)));
-        }
-      }
+      for (int i = 0; i < TC_FG / 2; i++)
+        dz1[i] = __fmul2_rn(__fadd2_rn(f2(ndh1[2 * i], ndh1[2 * i + 1]), f2(ndh1b[2 * i], ndh1b[2 * i + 1])), f2(dt[2 * i], dt[2 * i + 1]));
       TR(12);
       mbar_wait(bar2, ph);  // G2 has consumed h1^T and dz2^T
       TR(13);
@@ -893,6 +867,7 @@ __device__ __forceinline__ void grid_barrier(unsigned long long* ctr) {
   __syncthreads();
 }
 constexpr int FT_EL = 64;  // elements per reduction pass (x 4 partial groups = 256 threads)
+constexpr int FT_BATCH = 10;  // partials per thread in flight in the slab reduction
 // -DFT_TRACE: clock stamps of the tail's phases, printed by thread 0 of the first and the last CTA (development aid)
 #ifdef FT_TRACE
 __device__ __forceinline__ long long gtime() { long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
@@ -952,9 +927,6 @@ __device__ __noinline__ void fused_tail(const UpdateArgs& a, float* scratch, con
       if (critic) c_lo = a.tc_actor_ctas; else c_hi = a.tc_actor_ctas;
       // FT_BATCH partials requested before the first is added (one L2 round trip per batch); same summation order as the
       // plain loop: adding the +0.0f of a padded slot changes nothing
-#ifndef FT_BATCH
-#define FT_BATCH 10
-#endif
       for (int c0 = c_lo + g; c0 < c_hi; c0 += 4 * FT_BATCH) {
         float v[FT_BATCH];
 #pragma unroll
@@ -1244,16 +1216,11 @@ cudaError_t kernels_init_update_tc() {
 
 // Chooses the tensor-core kernel for this minibatch when it applies (parameter image present) and fills
 // in the launch geometry; CRL_NO_TC=1 keeps the FFMA kernel.
-#ifndef TC_ACTOR_COST
-#define TC_ACTOR_COST 1.15
-#endif
 int loss_grad_tc_plan(UpdateArgs* a, int sm_count, bool full_grid) {
-  static int disabled = -1, actor_share = -1;
+  static int disabled = -1;
   if (disabled < 0) {
     const char* e = getenv("CRL_NO_TC");
     disabled = (e && atoi(e) != 0) ? 1 : 0;
-    const char* s = getenv("CRL_TC_ACTOR_CTAS");
-    actor_share = s ? atoi(s) : 0;
   }
   a->tc_actor_ctas = 0;
   // A2C: the actor's advantage needs the critic's output, which lives in other CTAs; only when the recorded values
@@ -1263,19 +1230,20 @@ int loss_grad_tc_plan(UpdateArgs* a, int sm_count, bool full_grid) {
   int grid = (2 * n_tiles < sm_count && !full_grid) ? 2 * n_tiles : sm_count;
   grid &= ~1;
   if (grid < 2) grid = 2;
-  // An actor tile (two heads, softmax, entropy) costs TC_ACTOR_COST x a critic tile (clock stamps of the -DTC_TRACE
-  // build are perturbed by the stamps and show them equal; the A/B runs of CRL_TC_ACTOR_CTAS say 79 of 148), and every CTA runs a whole number of tiles: pick the split that minimises the
-  // slower side.
+  // An actor tile (two heads, softmax, entropy) costs 1.15 x a critic tile: the clock stamps of the -DTC_TRACE build
+  // are perturbed by the stamps and show them equal, while the timed splits of DESIGN.md §9 are fastest at 79 of 148
+  // CTAs on the actor, which this cost picks for the benchmark's 1024 tiles. Every CTA runs a whole number of tiles:
+  // pick the split that minimises the slower side.
+  constexpr double actor_cost = 1.15;
   int na = grid / 2;
   {
     double best = 1e30;
     for (int cand = 1; cand < grid; cand++) {
-      const double ta = TC_ACTOR_COST * ((n_tiles + cand - 1) / cand), tc = (double)((n_tiles + (grid - cand) - 1) / (grid - cand));
+      const double ta = actor_cost * ((n_tiles + cand - 1) / cand), tc = (double)((n_tiles + (grid - cand) - 1) / (grid - cand));
       const double cost = ta > tc ? ta : tc;
       if (cost < best - 1e-9) { best = cost; na = cand; }
     }
   }
-  if (actor_share > 0 && actor_share < grid && grid == (sm_count & ~1)) na = actor_share;
   a->grid_loss = grid;
   a->tc_actor_ctas = na;
   return 1;
@@ -1283,8 +1251,6 @@ int loss_grad_tc_plan(UpdateArgs* a, int sm_count, bool full_grid) {
 
 template <int ENV> static cudaError_t launch_fused_t(const UpdateArgs& a, cudaStream_t s) {
   // the grid barriers of the fused tail need every CTA resident: cooperative launch (grid <= SM count, 1 CTA per SM)
-  static int no_coop = -1;
-  if (no_coop < 0) { const char* e = getenv("CRL_NO_COOP"); no_coop = (e && atoi(e) != 0) ? 1 : 0; }
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)a.grid_loss);
   cfg.blockDim = dim3(TC_THREADS);
@@ -1294,7 +1260,7 @@ template <int ENV> static cudaError_t launch_fused_t(const UpdateArgs& a, cudaSt
   at[0].id = cudaLaunchAttributeCooperative;
   at[0].val.cooperative = 1;
   cfg.attrs = at;
-  cfg.numAttrs = no_coop ? 0 : 1;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, loss_grad_tc_kernel<ENV>, a);
 }
 

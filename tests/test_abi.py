@@ -81,6 +81,22 @@ def test_no_cpu_fallback_without_a_gpu(crl, abi):
     assert b"divisible" in lib.crl_last_error()
 
 
+ENV_SWITCHES = {"CRL_NO_TC", "CRL_EXACT", "CRL_MULTI_EXACT", "CRL_NO_GRAPH", "CRL_NO_P2P", "CRL_P2P_TIMEOUT_MS",
+                "CRL_NCCL_LIB"}
+
+
+def test_library_reads_exactly_the_documented_environment_switches():
+    """every environment variable the native library reads is one of the switches README.md documents, and each is there"""
+    csrc = os.path.join(ROOT, "cleanrl.jl_b200", "csrc")
+    read = set()
+    for f in os.listdir(csrc):
+        read |= set(re.findall(r'getenv\(\s*"(\w+)"\s*\)', open(os.path.join(csrc, f)).read()))
+    assert read == ENV_SWITCHES
+    readme = open(os.path.join(ROOT, "README.md")).read()
+    for name in sorted(ENV_SWITCHES):
+        assert "`%s" % name in readme, name
+
+
 def test_product_package_never_imports_the_oracle():
     pkg = os.path.join(ROOT, "cleanrl.jl_b200")
     for dirpath, _, files in os.walk(pkg):

@@ -1,4 +1,4 @@
-"""GAE HBM sweep: achieved GB/s of crl_gae_raw at T=128 for several N (and kernel variants via CRL_GAE_VARIANT)."""
+"""GAE HBM sweep: achieved GB/s of crl_gae_raw at T=128 for several N."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -19,5 +19,5 @@ for N in (1 << 18, 1 << 20, 1 << 21):
     for _ in range(10): launch()
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / 10
-    print("variant", os.environ.get("CRL_GAE_VARIANT", "0"), "N", N, "ms %.4f" % ms, "GB/s %.0f" % ((17 * T * N + 5 * N) / ms / 1e6))
+    print("N", N, "ms %.4f" % ms, "GB/s %.0f" % ((17 * T * N + 5 * N) / ms / 1e6))
     del v, r, d, adv, ret
