@@ -9,7 +9,7 @@ nothing — the library is dlopen'ed on first use and there is no CPU fallback.
 from . import _abi  # noqa: F401
 from .config import PPOConfig, argparse_struct  # noqa: F401
 
-__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "argparse_struct", "ppo", "a2c", "dqn", "PPOHandle", "Networks", "Logger",
+__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "DDPGConfig", "argparse_struct", "ppo", "a2c", "dqn", "ddpg", "PPOHandle", "Networks", "Logger",
            "ConfigParser"]
 
 
@@ -31,7 +31,16 @@ def dqn(*args, **kwargs):
     return _dqn(*args, **kwargs)
 
 
+def ddpg(*args, **kwargs):
+    """Vectorised DDPG on Pendulum (pinned to include/cleanrl_ddpg.h, not ddpg.jl); see ddpg_algo.py"""
+    from .ddpg_algo import ddpg as _ddpg
+    return _ddpg(*args, **kwargs)
+
+
 def __getattr__(name):
+    if name == "DDPGConfig":
+        from .ddpg_algo import DDPGConfig
+        return DDPGConfig
     if name == "DQNConfig":
         from .dqn_algo import DQNConfig
         return DQNConfig

@@ -89,3 +89,30 @@ def make_dqn_config(num_envs=1, buffer_size=10_000, min_buff_size=200, batch_siz
     return crl_dqn_config(C.sizeof(crl_dqn_config), num_envs, buffer_size, min_buff_size, batch_size, train_freq,
                           target_net_freq, max_episode_steps, device, 0, lr, gamma, epsilon_start, epsilon_end,
                           epsilon_duration, seed)
+
+
+# ---- DDPG (include/cleanrl_ddpg.h) ----------------------------------------------------------------------------
+CRL_DDPG_ACTOR_PARAMS = 4481
+CRL_DDPG_CRITIC_PARAMS = 4545
+
+
+class crl_ddpg_config(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_int32), ("num_envs", C.c_int32), ("buffer_size", C.c_int32), ("learning_starts", C.c_int32),
+        ("batch_size", C.c_int32), ("train_freq", C.c_int32), ("policy_frequency", C.c_int32),
+        ("max_episode_steps", C.c_int32), ("device", C.c_int32), ("_pad", C.c_int32),
+        ("gamma", C.c_double), ("tau", C.c_double), ("lr", C.c_double), ("exploration_noise", C.c_double), ("seed", C.c_uint64),
+    ]
+
+
+class crl_ddpg_stats(C.Structure):
+    _fields_ = [("critic_loss", C.c_double), ("actor_loss", C.c_double), ("sum_return", C.c_double), ("sum_length", C.c_double),
+                ("episodes", C.c_int64), ("learn_steps", C.c_int64), ("actor_steps", C.c_int64), ("iterations", C.c_int64),
+                ("kernel_launches", C.c_int64)]
+
+
+def make_ddpg_config(num_envs=1, buffer_size=1_000_000, learning_starts=25_000, batch_size=256, train_freq=1, policy_frequency=2,
+                     max_episode_steps=200, device=0, gamma=0.99, tau=0.005, lr=3e-4, exploration_noise=0.1, seed=1):
+    """crl_ddpg_config with CleanRL's ddpg_continuous_action.py defaults (PendulumEnv() max_steps = 200)."""
+    return crl_ddpg_config(C.sizeof(crl_ddpg_config), num_envs, buffer_size, learning_starts, batch_size, train_freq,
+                           policy_frequency, max_episode_steps, device, 0, gamma, tau, lr, exploration_noise, seed)

@@ -79,6 +79,21 @@ SIGNATURES = {
     "crl_tb_close": (C.c_int, [V]),
 }
 
+# every symbol include/cleanrl_ddpg.h declares (the DDPG handle and its raw kernels)
+DDPG_SIGNATURES = {
+    "crl_ddpg_create": (C.c_int, [C.POINTER(_abi.crl_ddpg_config), C.POINTER(V)]),
+    "crl_ddpg_destroy": (C.c_int, [V]),
+    "crl_ddpg_set_params": (C.c_int, [V, V, I32, V, I32]),
+    "crl_ddpg_get_params": (C.c_int, [V, V, V, V, V]),
+    "crl_ddpg_get_adam_state": (C.c_int, [V, V, V, V, V, V]),
+    "crl_ddpg_reset": (C.c_int, [V]),
+    "crl_ddpg_run": (C.c_int, [V, I64, V]),
+    "crl_ddpg_read_buffer": (C.c_int, [V] * 8),
+    "crl_ddpg_forward_raw": (C.c_int, [V] * 6 + [I64, V]),
+    "crl_ddpg_critic_loss_raw": (C.c_int, [V, V, V, I32] + [V] * 5 + [F64, V, V, V]),
+    "crl_ddpg_actor_loss_raw": (C.c_int, [V, V, I32, V, V, V, V]),
+}
+
 
 def load():
     """dlopen the CUDA library and bind every entry point. Raises if it is not built."""
@@ -89,7 +104,7 @@ def load():
         raise CleanRLCudaError(-2, "%s is not built (run `python cleanrl.jl_b200/build.py` or "
                                    "__graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = C.CDLL(LIB_PATH, mode=C.RTLD_GLOBAL)
-    for name, (res, args) in SIGNATURES.items():
+    for name, (res, args) in list(SIGNATURES.items()) + list(DDPG_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError here = header/library mismatch
         fn.restype = res
         fn.argtypes = args

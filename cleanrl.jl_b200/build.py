@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libcleanrl_cuda.so")
-SOURCES = ["gae.cu", "rollout.cu", "update.cu", "update_tc.cu", "dqn.cu", "tblog.cu", "api.cu"]
+SOURCES = ["gae.cu", "rollout.cu", "update.cu", "update_tc.cu", "dqn.cu", "ddpg.cu", "tblog.cu", "api.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"] + os.environ.get("CRL_NVCC_EXTRA", "").split()
 
@@ -23,7 +23,7 @@ def needs_build():
     if not os.path.exists(OUT):
         return True
     t = os.path.getmtime(OUT)
-    deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "cleanrl_cuda.h")]
+    deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", h) for h in ("cleanrl_cuda.h", "cleanrl_ddpg.h")]
     return any(os.path.getmtime(d) > t for d in deps)
 
 

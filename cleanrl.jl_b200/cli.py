@@ -1,4 +1,4 @@
-"""Runner: `python -m cleanrl_jl_b200 {ppo,a2c,dqn} [--field value ...]`.
+"""Runner: `python -m cleanrl_jl_b200 {ppo,a2c,dqn,ddpg} [--field value ...]`.
 
 The reference leaves this wiring as a TODO ("Make individual file runners e.g experiments/run_ppo.(jl/sh)", README.md:24):
 `ConfigParser.argparse_struct` exists (config_parser.jl:18-40) but nothing calls it. Here every field of the algorithm's
@@ -19,14 +19,23 @@ def _configs():
     return {"ppo": PPOConfig, "a2c": A2CConfig, "dqn": DQNConfig}
 
 
+def _single_gpu_configs():
+    """algorithms with no multi-GPU path (DDPG on Pendulum: one GPU, include/cleanrl_ddpg.h)"""
+    from .ddpg_algo import DDPGConfig
+    return {"ddpg": DDPGConfig}
+
+
 def main(argv=None):
     argv = list(sys.argv[1:] if argv is None else argv)
     algos = _configs()
-    if not argv or argv[0] in ("-h", "--help") or argv[0] not in algos:
+    single = _single_gpu_configs()
+    if not argv or argv[0] in ("-h", "--help") or argv[0] not in {**algos, **single}:
         sys.stderr.write("usage: python -m cleanrl_jl_b200 {%s} [--<config field> <value> ...]\n"
+                         "       python -m cleanrl_jl_b200 {%s} [--<config field> <value> ...]   (one GPU)\n"
                          "       (every field of the algorithm's config struct is an option; --help after the algorithm lists them)\n"
-                         % ",".join(sorted(algos)))
+                         % (",".join(sorted(algos)), ",".join(sorted(single))))
         return 2
+    algos = {**algos, **single}
     from .config import argparse_struct
     algo = argv[0]
     config = argparse_struct(algos[algo](), argv[1:])
@@ -39,8 +48,8 @@ def main(argv=None):
         torch.cuda.set_device(local_rank)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     try:
-        from . import a2c, dqn, ppo
-        res = {"ppo": ppo, "a2c": a2c, "dqn": dqn}[algo](config)
+        from . import a2c, ddpg, dqn, ppo
+        res = {"ppo": ppo, "a2c": a2c, "dqn": dqn, "ddpg": ddpg}[algo](config)
     finally:
         if dist is not None:
             dist.destroy_process_group()

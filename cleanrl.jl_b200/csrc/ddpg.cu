@@ -1,0 +1,857 @@
+// ddpg.cu — vectorised DDPG on Pendulum behind the crl_ddpg_* entry points of include/cleanrl_ddpg.h: N Pendulum envs
+// stepping in lockstep with a deterministic actor plus Gaussian exploration noise, an HBM-resident ring replay buffer, and
+// one learning step (sample without replacement -> critic TD regression against the target nets -> Adam; on every
+// policy_frequency-th learning step the actor's -Q gradient through the just-updated critic -> Adam -> Polyak averaging of
+// both targets) every train_freq iterations.
+//
+// The reference's ddpg.jl trains on MuJoCo HalfCheetah through PyCall and is not part of this checkout; the semantics are
+// pinned by the header (CleanRL-Python's ddpg_continuous_action.py with 64-wide nets on Pendulum), not by ddpg.jl.
+//
+// Both nets are Dense(IN,64,relu) -> Dense(64,64,relu) -> Dense(64,1) (actor: IN = 3, then 2 tanh; critic: IN = 4 =
+// [obs; action]). Every kernel evaluates them out of shared memory with mlp_forward: register tiles of 4 neurons x 4
+// samples in the hidden layer, and every neuron is ONE fmaf chain over ascending k, so results do not depend on the tiling.
+//
+//   ddpg_act_kernel         32 envs per CTA of 256 threads. All threads evaluate the actor; warp 0 (one lane per env,
+//                           state in registers) draws the warm-up or noise action from Philox stream 5, steps Pendulum,
+//                           appends the transition at (ptr + step * N + env) % capacity and resets a finished env on the
+//                           spot. The parameters only change at a learning step, so ONE launch runs every iteration up
+//                           to the next learning step.
+//   ddpg_critic_fwd_kernel  learning step, critic part 1: CTA c owns samples 16c..16c+15 of the batch: gather, target
+//                           actor, target critic, TD target (Float64), critic forward, loss, backward deltas; what the
+//                           weight gradients need is written sample-major to a global scratch (L2-resident).
+//   ddpg_actor_fwd_kernel   actor part 1 on the same batch: actor forward, critic forward on [obs; mu(obs)], the
+//                           gradient of -mean Q back through the critic to the action input, then through the actor.
+//   ddpg_update_kernel<IN>  part 2 for either net: one thread per parameter sums its gradient over the batch in ascending
+//                           sample order (deterministic, no float atomics) and applies Adam in place.
+//   ddpg_polyak_kernel      theta' <- tau theta + (1 - tau) theta' for both targets, after the actor step only.
+// The raw entry points run the same kernels on rows the caller passes in (sample b = row b), with the gradient written
+// out instead of an Adam step, so that each can be compared with a reference on its own. Every decision that only
+// depends on counters (learn on this iteration?, actor step?, Adam's beta powers) is taken on the host, so a run is a
+// plain sequence of launches on one stream without any device-to-host read.
+#include <math.h>
+#include <stdlib.h>
+#include <string.h>
+
+#include <string>
+
+#include "../../include/cleanrl_ddpg.h"
+#include "device_math.cuh"
+#include "kernels.h"
+
+namespace {
+
+// ---- network geometry (the one place the widths live)
+constexpr int DD_D = 3, DD_A = 1, DD_H = 64;   // observation [cos th, sin th, thdot], torque, hidden width
+constexpr float DD_MAX_TORQUE = 2.0f;
+template <int IN> struct DNet {                 // flat Flux.params order, each W (out,in) column-major
+  static constexpr int W1 = 0, B1 = W1 + DD_H * IN, W2 = B1 + DD_H, B2 = W2 + DD_H * DD_H, W3 = B2 + DD_H, B3 = W3 + DD_H,
+                       P = B3 + 1, PP = (P + 3) & ~3;
+};
+using ANet = DNet<DD_D>;           // actor mu
+using CNet = DNet<DD_D + DD_A>;    // critic Q
+static_assert(ANet::P == CRL_DDPG_ACTOR_PARAMS && CNet::P == CRL_DDPG_CRITIC_PARAMS, "parameter counts");
+static_assert(ANet::W2 % 4 == 0 && CNet::W2 % 4 == 0, "128-bit weight loads of the hidden layer");
+
+constexpr uint32_t STREAM_DDPG_ACT = 5u, STREAM_DDPG_BATCH = 6u;
+constexpr int ACT_E = 32;                 // envs per CTA in ddpg_act_kernel
+constexpr int ACT_SP = ACT_E + 4;         // activation row stride (floats): rows stay 16-byte aligned
+constexpr int ACT_T = 256;                // threads of ddpg_act_kernel
+constexpr int ACT_MAX_STEPS = 1024;       // iterations per ddpg_act_kernel launch (bounds one launch's duration)
+constexpr int LEARN_B = 256;              // max batch size
+constexpr int LF_S = 16, LF_SP = LF_S + 4, LF_T = 256;   // learning forward kernels: samples per CTA, row stride, threads
+constexpr int LF_MAX_BLOCKS = LEARN_B / LF_S;
+constexpr int XS = 4;                     // row stride of the gathered inputs in the scratch (critic: 4, actor: 3 used)
+constexpr int LU_T = 256;                 // ddpg_update_kernel threads
+
+struct DdpgDev {               // device-resident scalars
+  double critic_loss, actor_loss;
+  double sum_return, sum_length;
+  unsigned long long episodes;
+};
+
+// global -> shared copy of one parameter vector of P floats (128-bit loads; cudaMalloc'ed source, 16-byte aligned dst)
+template <int P, int NT> __device__ __forceinline__ void load_params(const float* __restrict__ g, float* sp, int tid) {
+  const float4* g4 = reinterpret_cast<const float4*>(g);
+  float4* s4 = reinterpret_cast<float4*>(sp);
+  constexpr int N4 = P / 4, PER = (N4 + NT - 1) / NT;
+  float4 tmp[PER];   // every load is in flight before the first store
+#pragma unroll
+  for (int u = 0; u < PER; u++) if (tid + u * NT < N4) tmp[u] = g4[tid + u * NT];
+#pragma unroll
+  for (int u = 0; u < PER; u++) if (tid + u * NT < N4) s4[tid + u * NT] = tmp[u];
+  if (tid < P % 4) sp[N4 * 4 + tid] = g[N4 * 4 + tid];
+}
+
+// Dense(IN,64,relu) -> Dense(64,64,relu) -> Dense(64,1) for a tile of NS samples by the NT threads of the CTA (every
+// thread must call this: __syncthreads between the layers and at the end). p: parameters in shared memory (16-byte
+// aligned); xs [IN][SP] the inputs, h1/h2 [64][SP] the activations, out [SP] the head's pre-activation. A thread owns 4
+// consecutive samples of one first-layer neuron, then 4 neurons x 4 samples of the hidden layer (one 128-bit weight load
+// + one 128-bit activation load per k for 16 FMAs), then one sample of the head.
+template <int IN, int NS, int SP, int NT>
+__device__ __forceinline__ void mlp_forward(const float* __restrict__ p, const float* xs, float* h1, float* h2, float* out, int tid) {
+  using N = DNet<IN>;
+  constexpr int EQ = NS / 4;
+  static_assert(NS % 4 == 0 && SP % 4 == 0 && SP >= NS && NS <= NT, "tile geometry");
+  for (int w = tid; w < DD_H * EQ; w += NT) {
+    const int eq = w % EQ, j = w / EQ;
+    float4 acc = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+#pragma unroll
+    for (int k = 0; k < IN; k++) {
+      const float wt = p[N::W1 + j + DD_H * k];
+      const float4 x = *reinterpret_cast<const float4*>(xs + k * SP + 4 * eq);
+      acc.x = fmaf(wt, x.x, acc.x); acc.y = fmaf(wt, x.y, acc.y); acc.z = fmaf(wt, x.z, acc.z); acc.w = fmaf(wt, x.w, acc.w);
+    }
+    const float b = p[N::B1 + j];
+    *reinterpret_cast<float4*>(h1 + j * SP + 4 * eq) =
+        make_float4(fmaxf(acc.x + b, 0.0f), fmaxf(acc.y + b, 0.0f), fmaxf(acc.z + b, 0.0f), fmaxf(acc.w + b, 0.0f));
+  }
+  __syncthreads();
+  for (int w = tid; w < (DD_H / 4) * EQ; w += NT) {
+    const int eq = w % EQ, j = 4 * (w / EQ);
+    float acc[4][4];   // 16 independent scalar chains
+#pragma unroll
+    for (int n = 0; n < 4; n++)
+#pragma unroll
+      for (int c = 0; c < 4; c++) acc[n][c] = 0.0f;
+#pragma unroll 8
+    for (int k = 0; k < DD_H; k++) {
+      const float4 wv4 = *reinterpret_cast<const float4*>(p + N::W2 + j + DD_H * k);
+      const float4 hv4 = *reinterpret_cast<const float4*>(h1 + k * SP + 4 * eq);
+      const float wv[4] = {wv4.x, wv4.y, wv4.z, wv4.w}, hv[4] = {hv4.x, hv4.y, hv4.z, hv4.w};
+#pragma unroll
+      for (int n = 0; n < 4; n++)
+#pragma unroll
+        for (int c = 0; c < 4; c++) acc[n][c] = fmaf(wv[n], hv[c], acc[n][c]);
+    }
+#pragma unroll
+    for (int n = 0; n < 4; n++) {
+      const float b = p[N::B2 + j + n];
+      *reinterpret_cast<float4*>(h2 + (j + n) * SP + 4 * eq) =
+          make_float4(fmaxf(acc[n][0] + b, 0.0f), fmaxf(acc[n][1] + b, 0.0f), fmaxf(acc[n][2] + b, 0.0f), fmaxf(acc[n][3] + b, 0.0f));
+    }
+  }
+  __syncthreads();
+  if (tid < NS) {
+    float acc = 0.0f;
+#pragma unroll 16
+    for (int k = 0; k < DD_H; k++) acc = fmaf(p[N::W3 + k], h2[k * SP + tid], acc);
+    out[tid] = acc + p[N::B3];
+  }
+  __syncthreads();
+}
+
+// mu = 2 tanh(head), the torque limit of Pendulum
+__device__ __forceinline__ float actor_out(float u) { return DD_MAX_TORQUE * tanhf(u); }
+
+// Backward of Dense(IN,64,relu) -> Dense(64,64,relu) -> Dense(64,1) for the CTA's NS samples given d(head) per sample
+// in dout: exports x (rows 0..IN-1 of xs), h1, h2, dz2 and dz1 sample-major (neuron fastest) for samples b0 + i < B, and
+// leaves dz1 in z1s when it is not null (the actor step needs the critic's dz1 for the gradient of the action input).
+struct Scratch {
+  float *xT, *h1T, *h2T, *z1T, *z2T, *dT;   // [B][XS], [B][64] x4, [B]
+};
+template <int IN, int NS, int SP, int NT>
+__device__ __forceinline__ void mlp_backward(const float* __restrict__ p, const float* xs, const float* h1, const float* h2,
+                                             const float* dout, float* z2s, float* z1s, const Scratch& s, int b0, int B,
+                                             bool do_export, int tid) {
+  using N = DNet<IN>;
+  for (int w = tid; w < DD_H * NS; w += NT) {
+    const int k = w % DD_H, i = w / DD_H, b = b0 + i;
+    const float hv = h2[k * SP + i];
+    const float z = hv > 0.0f ? p[N::W3 + k] * dout[i] : 0.0f;   // relu'(0) = 0, as Flux
+    z2s[k * SP + i] = z;
+    if (do_export && b < B) { s.h1T[b * DD_H + k] = h1[k * SP + i]; s.h2T[b * DD_H + k] = hv; s.z2T[b * DD_H + k] = z; }
+  }
+  if (do_export && tid < NS && b0 + tid < B) {
+    const int b = b0 + tid;
+#pragma unroll
+    for (int c = 0; c < IN; c++) s.xT[b * XS + c] = xs[c * SP + tid];
+    s.dT[b] = dout[tid];
+  }
+  __syncthreads();
+  for (int w = tid; w < DD_H * NS; w += NT) {
+    const int k = w % DD_H, i = w / DD_H, b = b0 + i;
+    float acc = 0.0f;
+    const float* wc = p + N::W2 + DD_H * k;   // column k of W2: W2(j, k) for ascending j
+#pragma unroll 16
+    for (int j = 0; j < DD_H; j++) acc = fmaf(wc[j], z2s[j * SP + i], acc);
+    const float z = h1[k * SP + i] > 0.0f ? acc : 0.0f;
+    if (z1s) z1s[k * SP + i] = z;
+    if (do_export && b < B) s.z1T[b * DD_H + k] = z;
+  }
+  __syncthreads();
+}
+
+struct ActArgs {
+  const float* actor;
+  float* env_state; int* env_t; double* ep_ret; int* ep_len; uint32_t* resets;
+  float *b_obs, *b_next, *b_act, *b_rew; uint8_t* b_term;
+  DdpgDev* dev;
+  unsigned long long seed, it0;   // it0 = iteration number (1-based) of step 0 of this launch
+  long long learning_starts;
+  float sigma;                    // exploration_noise * max torque
+  int n_steps;
+  int N, C, ptr, max_steps;
+};
+
+// Warps 0-7 evaluate the actor for the CTA's 32 envs (skipped while every step of the launch is warm-up); warp 0 (one
+// lane per env) then draws the action, records the transition and advances its env.
+__global__ void __launch_bounds__(ACT_T, 1) ddpg_act_kernel(ActArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  constexpr int SP = ACT_SP;
+  float* p = smem;                        // [ANet::PP]
+  float* h1 = p + ANet::PP;               // [64][SP]
+  float* h2 = h1 + DD_H * SP;             // [64][SP]
+  float* uo = h2 + DD_H * SP;             // [SP]
+  float* xs = uo + SP;                    // [3][SP] current observation of the CTA's envs
+  const int tid = threadIdx.x;
+  const bool any_policy = (long long)(a.it0 + a.n_steps - 1) * a.N > a.learning_starts;
+  if (any_policy) load_params<ANet::P, ACT_T>(a.actor, p, tid);
+  const int n = blockIdx.x * ACT_E + tid;
+  const bool owner = tid < ACT_E, valid = owner && n < a.N;
+  const uint32_t gid = (uint32_t)n;       // Philox is keyed by the global env id
+  float st[2] = {0.0f, 0.0f};
+  int t = 0, len = 0;
+  double ret = 0.0;
+  uint32_t rc = 0;
+  if (valid) {
+    const float2 s2 = reinterpret_cast<const float2*>(a.env_state)[n];
+    st[0] = s2.x; st[1] = s2.y;
+    t = a.env_t[n]; ret = a.ep_ret[n]; len = a.ep_len[n]; rc = a.resets[n];
+  }
+  for (int s = 0; s < a.n_steps; s++) {
+    const unsigned long long it = a.it0 + (unsigned long long)s;
+    const bool warm = (long long)it * a.N <= a.learning_starts;   // uniform over the grid
+    float obs[DD_D];
+    env_obs<CRL_ENV_PENDULUM>(st, obs);
+    if (owner) {
+#pragma unroll
+      for (int k = 0; k < DD_D; k++) xs[k * SP + tid] = obs[k];
+    }
+    if (!warm) {
+      __syncthreads();
+      mlp_forward<DD_D, ACT_E, SP, ACT_T>(p, xs, h1, h2, uo, tid);   // mu(obs)
+    }
+    if (valid) {
+      uint32_t r[4];
+      philox_draw(a.seed, gid, it, STREAM_DDPG_ACT, r);
+      float act;
+      if (warm) {
+        act = __fmaf_rn(2.0f * DD_MAX_TORQUE, (float)(r[0] >> 8) * (1.0f / 16777216.0f), -DD_MAX_TORQUE);   // U[-2, 2)
+      } else {
+        // Box-Muller standard normal from 24-bit uniforms (u1 in (0, 1]), as rng_action_normals
+        const float u1 = (float)((r[0] >> 8) + 1u) * (1.0f / 16777216.0f);
+        const float u2 = (float)(r[1] >> 8) * (1.0f / 16777216.0f);
+        const float z = sqrtf(-2.0f * logf(u1)) * cosf(6.283185307179586f * u2);
+        act = fmaf(a.sigma, z, actor_out(uo[tid]));
+        act = fminf(fmaxf(act, -DD_MAX_TORQUE), DD_MAX_TORQUE);
+      }
+      float rew;
+      bool done;
+      pendulum_step(st, t, act, a.max_steps, rew, done);
+      float nobs[DD_D];
+      env_obs<CRL_ENV_PENDULUM>(st, nobs);                         // next_obs before any reset
+      const long long slot = ((long long)a.ptr + (long long)s * a.N + n) % a.C;
+#pragma unroll
+      for (int k = 0; k < DD_D; k++) { a.b_obs[slot * DD_D + k] = obs[k]; a.b_next[slot * DD_D + k] = nobs[k]; }
+      a.b_act[slot] = act;
+      a.b_rew[slot] = rew;
+      a.b_term[slot] = done ? 1 : 0;
+      ret += (double)rew;
+      len += 1;
+      if (done) {
+        atomicAdd(&a.dev->episodes, 1ull);
+        atomicAdd(&a.dev->sum_return, ret);
+        atomicAdd(&a.dev->sum_length, (double)len);
+        ret = 0.0;
+        len = 0;
+        float u4[4];
+        rng_reset_uniforms(a.seed, gid, rc, u4);
+        pendulum_reset(st, t, u4);
+        rc += 1;
+      }
+    }
+    if (!warm) __syncthreads();   // uo and xs are rewritten by the next step
+  }
+  if (valid) {
+    a.ep_ret[n] = ret; a.ep_len[n] = len; a.env_t[n] = t; a.resets[n] = rc;
+    reinterpret_cast<float2*>(a.env_state)[n] = make_float2(st[0], st[1]);
+  }
+}
+
+// crl_ddpg_forward_raw: the acting kernel's actor forward pass (same mlp_forward instantiation, 32 samples per CTA) and
+// the critic on [obs; act] with the same tiling; rows past n are zero and not written back
+__global__ void __launch_bounds__(ACT_T, 1) ddpg_forward_raw_kernel(const float* actor, const float* critic, const float* obs,
+                                                                    const float* act, float* mu_out, float* q_out, int64_t n) {
+  extern __shared__ __align__(16) float smem[];
+  constexpr int SP = ACT_SP;
+  float* pa = smem;                       // [ANet::PP]
+  float* pc = pa + ANet::PP;              // [CNet::PP]
+  float* h1 = pc + CNet::PP;              // [64][SP]
+  float* h2 = h1 + DD_H * SP;             // [64][SP]
+  float* uo = h2 + DD_H * SP;             // [SP]
+  float* xs = uo + SP;                    // [4][SP]
+  const int tid = threadIdx.x;
+  load_params<ANet::P, ACT_T>(actor, pa, tid);
+  load_params<CNet::P, ACT_T>(critic, pc, tid);
+  const int64_t i = (int64_t)blockIdx.x * ACT_E + tid;
+  if (tid < ACT_E) {
+#pragma unroll
+    for (int k = 0; k < DD_D; k++) xs[k * SP + tid] = i < n ? obs[i * DD_D + k] : 0.0f;
+    xs[DD_D * SP + tid] = i < n ? act[i] : 0.0f;
+  }
+  __syncthreads();
+  mlp_forward<DD_D, ACT_E, SP, ACT_T>(pa, xs, h1, h2, uo, tid);
+  if (tid < ACT_E && i < n) mu_out[i] = actor_out(uo[tid]);
+  __syncthreads();
+  mlp_forward<DD_D + DD_A, ACT_E, SP, ACT_T>(pc, xs, h1, h2, uo, tid);
+  if (tid < ACT_E && i < n) q_out[i] = uo[tid];
+}
+
+struct LearnArgs {
+  const float *actor, *critic, *actor_tgt, *critic_tgt;
+  const float *b_obs, *b_next, *b_act, *b_rew; const uint8_t* b_term;
+  unsigned long long seed, learn_step;
+  double gamma;
+  int B, size;
+  int in_order;           // sample b is row b of the b_* arrays (raw entry points), not entry b of the keyed permutation
+  Scratch s;
+  double* loss_part;      // [LF_MAX_BLOCKS]
+};
+
+// sample(1:size, B, replace=false): the first B entries of a keyed permutation of [0, size), Philox stream 6 keyed by the
+// learning-step index (the critic and the actor step of one learning step see the same batch)
+__device__ __forceinline__ uint32_t batch_row(const LearnArgs& a, int b) {
+  if (a.in_order) return (uint32_t)b;
+  uint32_t keys[8];
+  philox_draw(a.seed, 0u, a.learn_step, STREAM_DDPG_BATCH, keys);
+  philox_draw(a.seed, 0x80000000u, a.learn_step, STREAM_DDPG_BATCH, keys + 4);
+  return perm_index((uint32_t)b, (uint32_t)a.size, perm_half_bits((uint32_t)a.size), keys);
+}
+
+// the squared errors (or Q-values) of the CTA's 16 samples summed in Float64 by lanes 0-15 of warp 0, in a fixed order
+__device__ __forceinline__ void block_part(double v, double* part) {
+#pragma unroll
+  for (int o = LF_S / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0x0000ffffu, v, o);
+  if (threadIdx.x == 0) part[blockIdx.x] = v;
+}
+
+__global__ void __launch_bounds__(LF_T) ddpg_critic_fwd_kernel(LearnArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  constexpr int SP = LF_SP;
+  float* pat = smem;                      // target actor
+  float* pct = pat + ANet::PP;            // target critic
+  float* pc = pct + CNet::PP;             // critic
+  float* h1 = pc + CNet::PP;              // [64][SP]
+  float* h2 = h1 + DD_H * SP;             // [64][SP]
+  float* z2 = h2 + DD_H * SP;             // [64][SP]
+  float* xin = z2 + DD_H * SP;            // [4][SP] obs, action
+  float* xn = xin + 4 * SP;               // [4][SP] next_obs, mu'(next_obs)
+  float* out = xn + 4 * SP;               // [SP]
+  float* dout = out + SP;                 // [SP]
+  __shared__ float s_rew[LF_S];
+  __shared__ int s_term[LF_S];
+  const int tid = threadIdx.x, B = a.B, b0 = blockIdx.x * LF_S;
+  // the gather (HBM latency) is issued first and completes under the parameter loads
+  float o[DD_D] = {0.0f, 0.0f, 0.0f}, nx[DD_D] = {0.0f, 0.0f, 0.0f}, act = 0.0f, rew = 0.0f;
+  int term = 0;
+  if (tid < LF_S && b0 + tid < B) {
+    const uint32_t idx = batch_row(a, b0 + tid);
+#pragma unroll
+    for (int k = 0; k < DD_D; k++) { o[k] = a.b_obs[idx * DD_D + k]; nx[k] = a.b_next[idx * DD_D + k]; }
+    act = a.b_act[idx]; rew = a.b_rew[idx]; term = a.b_term[idx];
+  }
+  load_params<ANet::P, LF_T>(a.actor_tgt, pat, tid);
+  load_params<CNet::P, LF_T>(a.critic_tgt, pct, tid);
+  load_params<CNet::P, LF_T>(a.critic, pc, tid);
+  if (tid < LF_S) {
+#pragma unroll
+    for (int k = 0; k < DD_D; k++) { xin[k * SP + tid] = o[k]; xn[k * SP + tid] = nx[k]; }
+    xin[DD_D * SP + tid] = act;
+    s_rew[tid] = rew; s_term[tid] = term;
+  }
+  __syncthreads();
+  mlp_forward<DD_D, LF_S, SP, LF_T>(pat, xn, h1, h2, out, tid);             // target_actor(next_obs)
+  if (tid < LF_S) xn[DD_D * SP + tid] = actor_out(out[tid]);
+  __syncthreads();
+  mlp_forward<DD_D + DD_A, LF_S, SP, LF_T>(pct, xn, h1, h2, out, tid);      // qf1_target(next_obs, mu'(next_obs))
+  double y = 0.0;
+  if (tid < LF_S) y = (double)s_rew[tid] + a.gamma * (1.0 - (double)s_term[tid]) * (double)out[tid];
+  mlp_forward<DD_D + DD_A, LF_S, SP, LF_T>(pc, xin, h1, h2, out, tid);      // qf1(obs, action)
+  if (tid < LF_S) {
+    const bool in = b0 + tid < B;
+    const double diff = (double)out[tid] - y;
+    dout[tid] = in ? (float)(2.0 * diff / (double)B) : 0.0f;               // d mse / d q
+    block_part(in ? diff * diff : 0.0, a.loss_part);
+  }
+  __syncthreads();
+  mlp_backward<DD_D + DD_A, LF_S, SP, LF_T>(pc, xin, h1, h2, dout, z2, nullptr, a.s, b0, B, true, tid);
+}
+
+__global__ void __launch_bounds__(LF_T) ddpg_actor_fwd_kernel(LearnArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  constexpr int SP = LF_SP;
+  float* pa = smem;                       // actor
+  float* pc = pa + ANet::PP;              // critic (as just updated)
+  float* h1a = pc + CNet::PP;             // [64][SP]
+  float* h2a = h1a + DD_H * SP;
+  float* h1c = h2a + DD_H * SP;
+  float* h2c = h1c + DD_H * SP;
+  float* z2 = h2c + DD_H * SP;
+  float* z1c = z2 + DD_H * SP;
+  float* xin = z1c + DD_H * SP;           // [4][SP] obs, mu(obs)
+  float* out = xin + 4 * SP;              // [SP]
+  float* dout = out + SP;                 // [SP]
+  const int tid = threadIdx.x, B = a.B, b0 = blockIdx.x * LF_S;
+  float o[DD_D] = {0.0f, 0.0f, 0.0f};
+  if (tid < LF_S && b0 + tid < B) {
+    const uint32_t idx = batch_row(a, b0 + tid);
+#pragma unroll
+    for (int k = 0; k < DD_D; k++) o[k] = a.b_obs[idx * DD_D + k];
+  }
+  load_params<ANet::P, LF_T>(a.actor, pa, tid);
+  load_params<CNet::P, LF_T>(a.critic, pc, tid);
+  if (tid < LF_S) {
+#pragma unroll
+    for (int k = 0; k < DD_D; k++) xin[k * SP + tid] = o[k];
+  }
+  __syncthreads();
+  mlp_forward<DD_D, LF_S, SP, LF_T>(pa, xin, h1a, h2a, out, tid);           // actor(obs)
+  float u = 0.0f;
+  if (tid < LF_S) { u = out[tid]; xin[DD_D * SP + tid] = actor_out(u); }
+  __syncthreads();
+  mlp_forward<DD_D + DD_A, LF_S, SP, LF_T>(pc, xin, h1c, h2c, out, tid);    // qf1(obs, actor(obs))
+  if (tid < LF_S) {
+    const bool in = b0 + tid < B;
+    dout[tid] = in ? (float)(-1.0 / (double)B) : 0.0f;                     // d(-mean Q) / dQ
+    block_part(in ? (double)out[tid] : 0.0, a.loss_part);
+  }
+  __syncthreads();
+  // through the critic (its gradient is not kept) to the action input: dL/da = sum_j W1c(j, action) dz1c(j)
+  mlp_backward<DD_D + DD_A, LF_S, SP, LF_T>(pc, xin, h1c, h2c, dout, z2, z1c, a.s, b0, B, false, tid);
+  if (tid < LF_S) {
+    float da = 0.0f;
+#pragma unroll 16
+    for (int j = 0; j < DD_H; j++) da = fmaf(pc[CNet::W1 + j + DD_H * DD_D], z1c[j * SP + tid], da);
+    // d(2 tanh u)/du = 2 sech^2 u, from cosh: 1 - tanh^2 would cancel where the head saturates
+    const float ch = coshf(u);
+    dout[tid] = b0 + tid < B ? da * (DD_MAX_TORQUE / (ch * ch)) : 0.0f;
+  }
+  __syncthreads();
+  mlp_backward<DD_D, LF_S, SP, LF_T>(pa, xin, h1a, h2a, dout, z2, nullptr, a.s, b0, B, true, tid);
+}
+
+struct UpdArgs {
+  float *params, *m, *v;
+  float* grads_out;        // non-null: write the gradient and leave params, m, v alone (raw entry points)
+  Scratch s;
+  const double* loss_part;
+  int n_parts, B;
+  double loss_sign;        // +1: critic (mean squared error), -1: actor (-mean Q)
+  double* loss_out;
+  double lr, bp1, bp2;     // beta1^t, beta2^t of Adam, kept on the host
+};
+
+// One thread per parameter of a DNet<IN>: its gradient summed over the batch in ascending sample order (one fmaf chain),
+// then Flux.Adam / torch.optim.Adam in the form of dqn_adam: Float64 scalars, Float32 state.
+template <int IN>
+__global__ void __launch_bounds__(LU_T) ddpg_update_kernel(UpdArgs a) {
+  using N = DNet<IN>;
+  const int i = blockIdx.x * LU_T + threadIdx.x;
+  if (i == 0) {
+    double sum = 0.0;
+    for (int c = 0; c < a.n_parts; c++) sum += a.loss_part[c];
+    *a.loss_out = a.loss_sign * sum / (double)a.B;
+  }
+  if (i >= N::P) return;
+  const int B = a.B;
+  const float *u, *w = nullptr;   // gradient = sum_b u[b * us] * w[b * ws] (w == nullptr: sum_b u[b * us])
+  int us, ws = 0;
+  if (i < N::B1) { u = a.s.z1T + (i % DD_H); us = DD_H; w = a.s.xT + i / DD_H; ws = XS; }
+  else if (i < N::W2) { u = a.s.z1T + (i - N::B1); us = DD_H; }
+  else if (i < N::B2) { const int r = i - N::W2; u = a.s.z2T + r % DD_H; us = DD_H; w = a.s.h1T + r / DD_H; ws = DD_H; }
+  else if (i < N::W3) { u = a.s.z2T + (i - N::B2); us = DD_H; }
+  else if (i < N::B3) { u = a.s.dT; us = 1; w = a.s.h2T + (i - N::W3); ws = DD_H; }
+  else { u = a.s.dT; us = 1; }
+  float g = 0.0f;
+  if (w) {
+#pragma unroll 8
+    for (int b = 0; b < B; b++) g = fmaf(__ldg(u + b * us), __ldg(w + b * ws), g);
+  } else {
+#pragma unroll 8
+    for (int b = 0; b < B; b++) g += __ldg(u + b * us);
+  }
+  if (a.grads_out) { a.grads_out[i] = g; return; }
+  const double b1 = 0.9, b2 = 0.999, eps = 1e-8;
+  const float m0 = a.m[i], v0 = a.v[i], p0 = a.params[i];
+  const double c1 = 1.0 - a.bp1, c2 = 1.0 - a.bp2;
+  const float mt = (float)__dadd_rn(__dmul_rn(b1, (double)m0), __dmul_rn(1.0 - b1, (double)g));
+  const float vt = (float)__dadd_rn(__dmul_rn(b2, (double)v0), __dmul_rn(__dmul_rn(1.0 - b2, (double)g), (double)g));
+  const double den = __dadd_rn(sqrt(__ddiv_rn((double)vt, c2)), eps);
+  const float step = (float)__dmul_rn(__ddiv_rn(__ddiv_rn((double)mt, c1), den), a.lr);
+  a.m[i] = mt;
+  a.v[i] = vt;
+  a.params[i] = __fsub_rn(p0, step);
+}
+
+// theta' <- tau theta + (1 - tau) theta' for the actor (i < ANet::P) and the critic, in Float64 and rounded once
+__global__ void __launch_bounds__(256) ddpg_polyak_kernel(const float* actor, float* actor_tgt, const float* critic, float* critic_tgt, double tau) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const float* p = i < ANet::P ? actor + i : critic + (i - ANet::P);
+  float* t = i < ANet::P ? actor_tgt + i : critic_tgt + (i - ANet::P);
+  if (i >= ANet::P + CNet::P) return;
+  *t = (float)__dadd_rn(__dmul_rn(tau, (double)*p), __dmul_rn(1.0 - tau, (double)*t));
+}
+
+__global__ void ddpg_reset_kernel(int N, unsigned long long seed, float* env_state, int* env_t, double* ep_ret, int* ep_len, uint32_t* resets) {
+  const int n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= N) return;
+  float u4[4], st[2];
+  int t;
+  rng_reset_uniforms(seed, (uint32_t)n, 0, u4);
+  pendulum_reset(st, t, u4);
+  env_state[2 * n] = st[0]; env_state[2 * n + 1] = st[1];
+  env_t[n] = t; ep_ret[n] = 0.0; ep_len[n] = 0; resets[n] = 1;
+}
+
+constexpr size_t ACT_SMEM = (ANet::PP + (2 * DD_H + 1 + DD_D) * ACT_SP) * sizeof(float);
+constexpr size_t FWD_RAW_SMEM = (ANet::PP + CNet::PP + (2 * DD_H + 1 + 4) * ACT_SP) * sizeof(float);
+constexpr size_t CF_SMEM = (ANet::PP + 2 * CNet::PP + (3 * DD_H + 8 + 2) * LF_SP) * sizeof(float);
+constexpr size_t AF_SMEM = (ANet::PP + CNet::PP + (6 * DD_H + 4 + 2) * LF_SP) * sizeof(float);
+static_assert(ACT_SMEM <= 227 * 1024 && FWD_RAW_SMEM <= 227 * 1024 && CF_SMEM <= 227 * 1024 && AF_SMEM <= 227 * 1024, "ddpg shared memory");
+constexpr size_t SCRATCH_FLOATS = (size_t)LEARN_B * (XS + 4 * DD_H + 1);
+
+int dfail(int code, const std::string& msg) { return crl_internal_fail(code, msg.c_str()); }
+#define DCK(call)                                                                                           \
+  do {                                                                                                      \
+    cudaError_t e__ = (call);                                                                               \
+    if (e__ != cudaSuccess)                                                                                 \
+      return dfail(CRL_ERR_CUDA, std::string(#call) + " failed: " + cudaGetErrorString(e__) + " (ddpg.cu)"); \
+  } while (0)
+
+template <typename T> cudaError_t dzalloc(T** p, size_t n) {
+  cudaError_t e = cudaMalloc(reinterpret_cast<void**>(p), (n ? n : 1) * sizeof(T));
+  if (e != cudaSuccess) return e;
+  return cudaMemset(*p, 0, (n ? n : 1) * sizeof(T));
+}
+
+Scratch carve(float* base) {
+  Scratch s;
+  s.h1T = base; s.h2T = s.h1T + LEARN_B * DD_H; s.z1T = s.h2T + LEARN_B * DD_H; s.z2T = s.z1T + LEARN_B * DD_H;
+  s.xT = s.z2T + LEARN_B * DD_H; s.dT = s.xT + LEARN_B * XS;
+  return s;
+}
+
+cudaError_t set_smem_attrs() {
+  cudaError_t e = cudaFuncSetAttribute(ddpg_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ACT_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ddpg_forward_raw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FWD_RAW_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ddpg_critic_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CF_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ddpg_actor_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AF_SMEM);
+  return e;
+}
+
+// the two kernels of one net's step: forward + deltas, then the reduction with Adam (grads_out == nullptr) or without
+cudaError_t launch_net_step(bool critic, const LearnArgs& l, UpdArgs u, cudaStream_t s) {
+  const int fwd_blocks = (l.B + LF_S - 1) / LF_S;
+  if (critic) ddpg_critic_fwd_kernel<<<fwd_blocks, LF_T, CF_SMEM, s>>>(l);
+  else ddpg_actor_fwd_kernel<<<fwd_blocks, LF_T, AF_SMEM, s>>>(l);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  u.s = l.s; u.loss_part = l.loss_part; u.n_parts = fwd_blocks; u.B = l.B; u.loss_sign = critic ? 1.0 : -1.0;
+  if (critic) ddpg_update_kernel<DD_D + DD_A><<<(CNet::P + LU_T - 1) / LU_T, LU_T, 0, s>>>(u);
+  else ddpg_update_kernel<DD_D><<<(ANet::P + LU_T - 1) / LU_T, LU_T, 0, s>>>(u);
+  return cudaGetLastError();
+}
+
+}  // namespace
+
+struct crl_ddpg_ctx {
+  crl_ddpg_config cfg;
+  cudaStream_t stream;
+  float *actor, *critic, *actor_tgt, *critic_tgt, *am, *av, *cm, *cv;
+  float* env_state; int* env_t; double* ep_ret; int* ep_len; uint32_t* resets;
+  float *b_obs, *b_next, *b_act, *b_rew; uint8_t* b_term;
+  DdpgDev* dev;
+  float* scratch;
+  double* loss_part;
+  double abp1, abp2, cbp1, cbp2;   // beta1^t, beta2^t of the actor's and the critic's Adam
+  int size, ptr;
+  long long it, learn_steps, actor_steps, launches;
+  bool params_set, reset_done;
+};
+
+static int ddpg_validate(const crl_ddpg_config* cfg) {
+  if (cfg->struct_size != (int32_t)sizeof(crl_ddpg_config)) return dfail(CRL_ERR_INVALID, "crl_ddpg_config.struct_size mismatch");
+  if (cfg->num_envs < 1 || cfg->buffer_size < cfg->num_envs) return dfail(CRL_ERR_INVALID, "need 1 <= num_envs <= buffer_size");
+  if (cfg->batch_size < 1 || cfg->batch_size > LEARN_B) return dfail(CRL_ERR_INVALID, "batch_size must be in [1, 256]");
+  if (cfg->train_freq < 1 || cfg->policy_frequency < 1 || cfg->max_episode_steps < 1)
+    return dfail(CRL_ERR_INVALID, "train_freq, policy_frequency and max_episode_steps must be positive");
+  if (!(cfg->tau > 0.0 && cfg->tau <= 1.0)) return dfail(CRL_ERR_INVALID, "tau must be in (0, 1]");
+  if (cfg->learning_starts < 0) return dfail(CRL_ERR_INVALID, "learning_starts must be >= 0");
+  if (!(cfg->exploration_noise >= 0.0) || !(cfg->lr > 0.0)) return dfail(CRL_ERR_INVALID, "need exploration_noise >= 0 and lr > 0");
+  return CRL_OK;
+}
+
+static int ddpg_device_check(int device) {
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return dfail(CRL_ERR_CUDA, "no CUDA device: libcleanrl_cuda has no CPU fallback");
+  if (device < 0 || device >= ndev) return dfail(CRL_ERR_INVALID, "device ordinal out of range");
+  cudaDeviceProp prop;
+  DCK(cudaGetDeviceProperties(&prop, device));
+  if (prop.major != 10) return dfail(CRL_ERR_CUDA, "libcleanrl_cuda is built for sm_100a only");
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_create(const crl_ddpg_config* cfg, crl_ddpg_ctx** out) {
+  if (!cfg || !out) return dfail(CRL_ERR_INVALID, "NULL argument");
+  *out = nullptr;
+  if (int rc = ddpg_validate(cfg)) return rc;
+  if (int rc = ddpg_device_check(cfg->device)) return rc;
+  DCK(cudaSetDevice(cfg->device));
+  crl_ddpg_ctx* c = new crl_ddpg_ctx();
+  memset(c, 0, sizeof(*c));
+  // from here on a failure must release what was allocated so far (crl_ddpg_destroy skips null members)
+#define DCKC(call)                                                                                            \
+  do {                                                                                                        \
+    cudaError_t e__ = (call);                                                                                 \
+    if (e__ != cudaSuccess) {                                                                                 \
+      crl_ddpg_destroy(c);                                                                                    \
+      return dfail(CRL_ERR_CUDA, std::string(#call) + " failed: " + cudaGetErrorString(e__) + " (ddpg.cu)"); \
+    }                                                                                                         \
+  } while (0)
+  c->cfg = *cfg;
+  const size_t N = cfg->num_envs, C = cfg->buffer_size;
+  DCKC(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
+  DCKC(dzalloc(&c->actor, ANet::PP)); DCKC(dzalloc(&c->actor_tgt, ANet::PP)); DCKC(dzalloc(&c->am, ANet::P)); DCKC(dzalloc(&c->av, ANet::P));
+  DCKC(dzalloc(&c->critic, CNet::PP)); DCKC(dzalloc(&c->critic_tgt, CNet::PP)); DCKC(dzalloc(&c->cm, CNet::P)); DCKC(dzalloc(&c->cv, CNet::P));
+  DCKC(dzalloc(&c->env_state, 2 * N)); DCKC(dzalloc(&c->env_t, N)); DCKC(dzalloc(&c->ep_ret, N)); DCKC(dzalloc(&c->ep_len, N));
+  DCKC(dzalloc(&c->resets, N));
+  DCKC(dzalloc(&c->b_obs, DD_D * C)); DCKC(dzalloc(&c->b_next, DD_D * C)); DCKC(dzalloc(&c->b_act, C)); DCKC(dzalloc(&c->b_rew, C));
+  DCKC(dzalloc(&c->b_term, C)); DCKC(dzalloc(&c->dev, 1));
+  DCKC(dzalloc(&c->scratch, SCRATCH_FLOATS)); DCKC(dzalloc(&c->loss_part, LF_MAX_BLOCKS));
+  DCKC(set_smem_attrs());
+#undef DCKC
+  *out = c;
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_destroy(crl_ddpg_ctx* c) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  cudaSetDevice(c->cfg.device);
+  if (c->stream) cudaStreamSynchronize(c->stream);
+  void* ptrs[] = {c->actor, c->critic, c->actor_tgt, c->critic_tgt, c->am, c->av, c->cm, c->cv, c->env_state, c->env_t, c->ep_ret,
+                  c->ep_len, c->resets, c->b_obs, c->b_next, c->b_act, c->b_rew, c->b_term, c->dev, c->scratch, c->loss_part};
+  for (void* p : ptrs) if (p) cudaFree(p);
+  if (c->stream) cudaStreamDestroy(c->stream);
+  delete c;
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_set_params(crl_ddpg_ctx* c, const float* actor, int32_t n_actor, const float* critic, int32_t n_critic) {
+  if (!c || !actor || !critic) return dfail(CRL_ERR_INVALID, "NULL argument");
+  if (n_actor != ANet::P || n_critic != CNet::P) return dfail(CRL_ERR_INVALID, "DDPG parameter vectors must have 4481 (actor) and 4545 (critic) floats");
+  DCK(cudaSetDevice(c->cfg.device));
+  DCK(cudaMemcpyAsync(c->actor, actor, sizeof(float) * ANet::P, cudaMemcpyHostToDevice, c->stream));
+  DCK(cudaMemcpyAsync(c->critic, critic, sizeof(float) * CNet::P, cudaMemcpyHostToDevice, c->stream));
+  DCK(cudaMemcpyAsync(c->actor_tgt, c->actor, sizeof(float) * ANet::P, cudaMemcpyDeviceToDevice, c->stream));
+  DCK(cudaMemcpyAsync(c->critic_tgt, c->critic, sizeof(float) * CNet::P, cudaMemcpyDeviceToDevice, c->stream));
+  DCK(cudaMemsetAsync(c->am, 0, sizeof(float) * ANet::P, c->stream)); DCK(cudaMemsetAsync(c->av, 0, sizeof(float) * ANet::P, c->stream));
+  DCK(cudaMemsetAsync(c->cm, 0, sizeof(float) * CNet::P, c->stream)); DCK(cudaMemsetAsync(c->cv, 0, sizeof(float) * CNet::P, c->stream));
+  DdpgDev d;
+  memset(&d, 0, sizeof(d));
+  DCK(cudaMemcpyAsync(c->dev, &d, sizeof(d), cudaMemcpyHostToDevice, c->stream));
+  DCK(cudaStreamSynchronize(c->stream));
+  c->abp1 = c->cbp1 = 0.9; c->abp2 = c->cbp2 = 0.999;
+  c->params_set = true;
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_get_params(crl_ddpg_ctx* c, float* actor, float* critic, float* actor_target, float* critic_target) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  DCK(cudaSetDevice(c->cfg.device));
+  if (actor) DCK(cudaMemcpyAsync(actor, c->actor, sizeof(float) * ANet::P, cudaMemcpyDeviceToHost, c->stream));
+  if (critic) DCK(cudaMemcpyAsync(critic, c->critic, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->stream));
+  if (actor_target) DCK(cudaMemcpyAsync(actor_target, c->actor_tgt, sizeof(float) * ANet::P, cudaMemcpyDeviceToHost, c->stream));
+  if (critic_target) DCK(cudaMemcpyAsync(critic_target, c->critic_tgt, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->stream));
+  DCK(cudaStreamSynchronize(c->stream));
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_get_adam_state(crl_ddpg_ctx* c, float* actor_m, float* actor_v, float* critic_m, float* critic_v,
+                                               double* beta_pow) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  DCK(cudaSetDevice(c->cfg.device));
+  if (actor_m) DCK(cudaMemcpyAsync(actor_m, c->am, sizeof(float) * ANet::P, cudaMemcpyDeviceToHost, c->stream));
+  if (actor_v) DCK(cudaMemcpyAsync(actor_v, c->av, sizeof(float) * ANet::P, cudaMemcpyDeviceToHost, c->stream));
+  if (critic_m) DCK(cudaMemcpyAsync(critic_m, c->cm, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->stream));
+  if (critic_v) DCK(cudaMemcpyAsync(critic_v, c->cv, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->stream));
+  DCK(cudaStreamSynchronize(c->stream));
+  if (beta_pow) { beta_pow[0] = c->abp1; beta_pow[1] = c->abp2; beta_pow[2] = c->cbp1; beta_pow[3] = c->cbp2; }
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_reset(crl_ddpg_ctx* c) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  DCK(cudaSetDevice(c->cfg.device));
+  const int N = c->cfg.num_envs;
+  ddpg_reset_kernel<<<(N + 127) / 128, 128, 0, c->stream>>>(N, c->cfg.seed, c->env_state, c->env_t, c->ep_ret, c->ep_len, c->resets);
+  DCK(cudaGetLastError());
+  c->size = 0; c->ptr = 0; c->it = 0; c->learn_steps = 0; c->actor_steps = 0;   /* launches is a lifetime counter */
+  c->reset_done = true;
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_run(crl_ddpg_ctx* c, int64_t iterations, crl_ddpg_stats* stats) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  if (iterations < 0) return dfail(CRL_ERR_INVALID, "iterations must be >= 0");
+  if (!c->params_set) return dfail(CRL_ERR_STATE, "crl_ddpg_run called before crl_ddpg_set_params");
+  if (!c->reset_done) return dfail(CRL_ERR_STATE, "crl_ddpg_run called before crl_ddpg_reset");
+  DCK(cudaSetDevice(c->cfg.device));
+  const crl_ddpg_config& g = c->cfg;
+  const int N = g.num_envs, C = g.buffer_size;
+  // per-call episode aggregate: clear the three accumulators, keep the last losses
+  DCK(cudaMemsetAsync(&c->dev->sum_return, 0, sizeof(double) * 2 + sizeof(unsigned long long), c->stream));
+  const Scratch s = carve(c->scratch);
+  int64_t k = 0;
+  while (k < iterations) {
+    // One launch acts for every iteration up to (and including) the next learning step: the parameters are constant in
+    // between. Bounded by ACT_MAX_STEPS and by the ring capacity (steps of one launch must not share a slot).
+    ActArgs a;
+    a.actor = c->actor; a.env_state = c->env_state; a.env_t = c->env_t; a.ep_ret = c->ep_ret; a.ep_len = c->ep_len; a.resets = c->resets;
+    a.b_obs = c->b_obs; a.b_next = c->b_next; a.b_act = c->b_act; a.b_rew = c->b_rew; a.b_term = c->b_term; a.dev = c->dev;
+    a.seed = g.seed; a.it0 = (unsigned long long)(c->it + 1); a.learning_starts = g.learning_starts;
+    a.sigma = (float)(g.exploration_noise * (double)DD_MAX_TORQUE);
+    a.N = N; a.C = C; a.ptr = c->ptr; a.max_steps = g.max_episode_steps;
+    int ns = 0;
+    bool learn = false;
+    while (k < iterations && ns < ACT_MAX_STEPS && (long long)(ns + 1) * N <= (long long)C && !learn) {
+      c->it += 1;
+      k += 1;
+      ns += 1;
+      c->ptr = (int)(((long long)c->ptr + N) % C);
+      c->size = c->size + N > C ? C : c->size + N;
+      const long long gs = c->it * (long long)N;
+      learn = gs > (long long)g.learning_starts && c->it % g.train_freq == 0 && c->size >= g.batch_size;
+    }
+    a.n_steps = ns;
+    ddpg_act_kernel<<<(N + ACT_E - 1) / ACT_E, ACT_T, ACT_SMEM, c->stream>>>(a);
+    DCK(cudaGetLastError());
+    c->launches += 1;
+    if (!learn) continue;
+    LearnArgs l;
+    memset(&l, 0, sizeof(l));
+    l.actor = c->actor; l.critic = c->critic; l.actor_tgt = c->actor_tgt; l.critic_tgt = c->critic_tgt;
+    l.b_obs = c->b_obs; l.b_next = c->b_next; l.b_act = c->b_act; l.b_rew = c->b_rew; l.b_term = c->b_term;
+    l.seed = g.seed; l.learn_step = (unsigned long long)c->learn_steps; l.gamma = g.gamma; l.B = g.batch_size; l.size = c->size;
+    l.s = s; l.loss_part = c->loss_part;
+    UpdArgs u;
+    memset(&u, 0, sizeof(u));
+    u.params = c->critic; u.m = c->cm; u.v = c->cv; u.loss_out = &c->dev->critic_loss; u.lr = g.lr; u.bp1 = c->cbp1; u.bp2 = c->cbp2;
+    DCK(launch_net_step(true, l, u, c->stream));
+    c->cbp1 *= 0.9; c->cbp2 *= 0.999;
+    c->launches += 2;
+    c->learn_steps += 1;
+    if (c->learn_steps % g.policy_frequency == 0) {   // every policy_frequency-th learning step, against the updated critic
+      u.params = c->actor; u.m = c->am; u.v = c->av; u.loss_out = &c->dev->actor_loss; u.bp1 = c->abp1; u.bp2 = c->abp2;
+      DCK(launch_net_step(false, l, u, c->stream));
+      ddpg_polyak_kernel<<<(ANet::P + CNet::P + 255) / 256, 256, 0, c->stream>>>(c->actor, c->actor_tgt, c->critic, c->critic_tgt, g.tau);
+      DCK(cudaGetLastError());
+      c->abp1 *= 0.9; c->abp2 *= 0.999;
+      c->launches += 3;
+      c->actor_steps += 1;
+    }
+  }
+  if (stats) {
+    DdpgDev d;
+    DCK(cudaMemcpyAsync(&d, c->dev, sizeof(d), cudaMemcpyDeviceToHost, c->stream));
+    DCK(cudaStreamSynchronize(c->stream));
+    stats->critic_loss = d.critic_loss; stats->actor_loss = d.actor_loss; stats->sum_return = d.sum_return;
+    stats->sum_length = d.sum_length; stats->episodes = (int64_t)d.episodes; stats->learn_steps = c->learn_steps;
+    stats->actor_steps = c->actor_steps; stats->iterations = c->it; stats->kernel_launches = c->launches;
+  }
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_read_buffer(crl_ddpg_ctx* c, float* obs, float* action, float* reward, float* next_obs,
+                                            uint8_t* terminal, int32_t* size, int32_t* ptr) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  DCK(cudaSetDevice(c->cfg.device));
+  const size_t C = c->cfg.buffer_size;
+  if (obs) DCK(cudaMemcpyAsync(obs, c->b_obs, C * DD_D * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (next_obs) DCK(cudaMemcpyAsync(next_obs, c->b_next, C * DD_D * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (action) DCK(cudaMemcpyAsync(action, c->b_act, C * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (reward) DCK(cudaMemcpyAsync(reward, c->b_rew, C * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (terminal) DCK(cudaMemcpyAsync(terminal, c->b_term, C, cudaMemcpyDeviceToHost, c->stream));
+  DCK(cudaStreamSynchronize(c->stream));
+  if (size) *size = c->size;
+  if (ptr) *ptr = c->ptr;
+  return CRL_OK;
+}
+
+// ---- raw entry points (device pointers)
+static int ddpg_raw_device_check() {
+  int dev = 0;
+  DCK(cudaGetDevice(&dev));
+  if (int rc = ddpg_device_check(dev)) return rc;
+  DCK(set_smem_attrs());
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_forward_raw(const float* actor, const float* critic, const float* obs, const float* action,
+                                            float* mu_out, float* q_out, int64_t n, void* stream) {
+  if (n < 0 || (n > 0 && (!actor || !critic || !obs || !action || !mu_out || !q_out))) return dfail(CRL_ERR_INVALID, "NULL argument or n < 0");
+  if (((uintptr_t)actor | (uintptr_t)critic) % 16) return dfail(CRL_ERR_INVALID, "actor and critic must be 16-byte aligned");
+  if (n == 0) return CRL_OK;
+  if (int rc = ddpg_raw_device_check()) return rc;
+  const int64_t grid = (n + ACT_E - 1) / ACT_E;
+  if (grid > 0x7fffffff) return dfail(CRL_ERR_INVALID, "n too large");
+  ddpg_forward_raw_kernel<<<(unsigned)grid, ACT_T, FWD_RAW_SMEM, (cudaStream_t)stream>>>(actor, critic, obs, action, mu_out, q_out, n);
+  DCK(cudaGetLastError());
+  return CRL_OK;
+}
+
+// one net's step of the learning step on rows 0..B-1 (nothing sampled), gradient out instead of Adam
+static int ddpg_loss_raw(bool critic, LearnArgs& l, float* grads_out, double* loss_out, cudaStream_t s) {
+  if (l.B < 1 || l.B > LEARN_B) return dfail(CRL_ERR_INVALID, "B must be in [1, 256]");
+  if (int rc = ddpg_raw_device_check()) return rc;
+  float* scratch = nullptr;
+  double* dscratch = nullptr;
+  DCK(cudaMalloc(reinterpret_cast<void**>(&scratch), SCRATCH_FLOATS * sizeof(float)));
+  if (cudaMalloc(reinterpret_cast<void**>(&dscratch), LF_MAX_BLOCKS * sizeof(double)) != cudaSuccess) {
+    cudaFree(scratch);
+    return dfail(CRL_ERR_CUDA, "cudaMalloc failed (crl_ddpg loss raw)");
+  }
+  l.in_order = 1; l.size = l.B; l.s = carve(scratch); l.loss_part = dscratch;
+  UpdArgs u;
+  memset(&u, 0, sizeof(u));
+  u.grads_out = grads_out; u.loss_out = loss_out;
+  cudaError_t e = launch_net_step(critic, l, u, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);   // the scratch is freed below
+  cudaFree(scratch);
+  cudaFree(dscratch);
+  if (e != cudaSuccess) return dfail(CRL_ERR_CUDA, std::string("crl_ddpg loss raw failed: ") + cudaGetErrorString(e));
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_ddpg_critic_loss_raw(const float* actor_target, const float* critic, const float* critic_target, int32_t B,
+                                                const float* obs, const float* action, const float* reward, const float* next_obs,
+                                                const uint8_t* terminal, double gamma, float* grads_out, double* loss_out, void* stream) {
+  if (!actor_target || !critic || !critic_target || !obs || !action || !reward || !next_obs || !terminal || !grads_out || !loss_out)
+    return dfail(CRL_ERR_INVALID, "NULL argument");
+  if (((uintptr_t)actor_target | (uintptr_t)critic | (uintptr_t)critic_target) % 16)
+    return dfail(CRL_ERR_INVALID, "parameter vectors must be 16-byte aligned");
+  LearnArgs l;
+  memset(&l, 0, sizeof(l));
+  l.actor_tgt = actor_target; l.critic = critic; l.critic_tgt = critic_target;
+  l.b_obs = obs; l.b_act = action; l.b_rew = reward; l.b_next = next_obs; l.b_term = terminal; l.gamma = gamma; l.B = B;
+  return ddpg_loss_raw(true, l, grads_out, loss_out, (cudaStream_t)stream);
+}
+
+extern "C" CRL_API int crl_ddpg_actor_loss_raw(const float* actor, const float* critic, int32_t B, const float* obs, float* grads_out,
+                                               double* loss_out, void* stream) {
+  if (!actor || !critic || !obs || !grads_out || !loss_out) return dfail(CRL_ERR_INVALID, "NULL argument");
+  if (((uintptr_t)actor | (uintptr_t)critic) % 16) return dfail(CRL_ERR_INVALID, "parameter vectors must be 16-byte aligned");
+  LearnArgs l;
+  memset(&l, 0, sizeof(l));
+  l.actor = actor; l.critic = critic; l.b_obs = obs; l.B = B;
+  return ddpg_loss_raw(false, l, grads_out, loss_out, (cudaStream_t)stream);
+}

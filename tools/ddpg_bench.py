@@ -1,0 +1,141 @@
+"""Time crl_ddpg_run on one GPU and print one JSON line.
+
+Workload: 4,096 Pendulum envs, a 1,048,576-transition ring, batch 256, a learning step every iteration,
+policy_frequency 2, learning_starts 10,000; and the same with num_envs 1 (one learning step per env step, CleanRL's
+update-to-data ratio). Reported:
+  * env-steps/s and learner steps/s over a timed window of whole crl_ddpg_run calls (device synchronised around it,
+    after a warm-up that fills past learning_starts);
+  * us per acting launch and per learning step (critic pair; actor pair + Polyak on every second step), from CUDA events
+    of torch.profiler in a separate profiled run;
+  * the same learning step written in PyTorch eager on the same GPU at B = 256, for comparison;
+  * the card's name, power limit and max SM clock, read in the same call.
+Usage: python tools/ddpg_bench.py [--iters 2000] [--out path.json]"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"], capture_output=True, text=True)
+    name, power, clock = [x.strip() for x in q.stdout.strip().splitlines()[0].split(",")]
+    return {"gpu": name, "power_limit": power, "max_sm_clock": clock}
+
+
+def make(num_envs):
+    from cleanrl_jl_b200 import _abi
+    from cleanrl_jl_b200.ddpg_algo import DDPGHandle, init_ddpg_params
+    cfg = _abi.make_ddpg_config(num_envs=num_envs, buffer_size=1 << 20, learning_starts=10_000, batch_size=256, train_freq=1,
+                                policy_frequency=2, seed=1)
+    h = DDPGHandle(cfg)
+    h.set_params(*init_ddpg_params(1))
+    h.reset()
+    return h
+
+
+def timed(torch, num_envs, iters):
+    h = make(num_envs)
+    h.run(10_000 // num_envs + 64)            # warm-up: past learning_starts, every kernel launched
+    torch.cuda.synchronize()
+    st0 = h.run(0)
+    t0 = time.perf_counter()
+    st = h.run(iters)
+    torch.cuda.synchronize()
+    dt = time.perf_counter() - t0
+    h.close()
+    return {"num_envs": num_envs, "iterations": iters, "seconds": dt, "env_steps_per_s": iters * num_envs / dt,
+            "learner_steps_per_s": (st.learn_steps - st0.learn_steps) / dt}
+
+
+def profiled(torch, iters, out_dir):
+    """per-kernel device time from torch.profiler (CUDA activities) in a run of its own"""
+    from torch.profiler import ProfilerActivity, profile
+    h = make(4096)
+    h.run(10_000 // 4096 + 8)
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        st0 = h.run(0)
+        st = h.run(iters)
+        torch.cuda.synchronize()
+    learn = st.learn_steps - st0.learn_steps
+    h.close()
+    per = {}
+    for e in prof.key_averages():
+        if "ddpg" in e.key:
+            k = e.key.replace("void ", "").replace("(anonymous namespace)::", "").split("(")[0]
+            per[k] = per.get(k, 0.0) + e.device_time_total
+    act = sum(v for k, v in per.items() if "act_kernel" in k)
+    lrn = sum(v for k, v in per.items() if "act_kernel" not in k)
+    if out_dir:
+        os.makedirs(out_dir, exist_ok=True)
+        prof.export_chrome_trace(os.path.join(out_dir, "ddpg_trace.json"))
+    return {"us_per_acting_launch": act / iters, "us_per_learning_step": lrn / max(learn, 1),
+            "kernel_us_total": {k: round(v, 1) for k, v in per.items()}}
+
+
+def eager(torch, reps=200):
+    """the same learning step (critic step every time, actor step + Polyak every second) in PyTorch eager, B = 256"""
+    import copy
+    nn = torch.nn
+    dev = "cuda"
+    mlp = lambda i: nn.Sequential(nn.Linear(i, 64), nn.ReLU(), nn.Linear(64, 64), nn.ReLU(), nn.Linear(64, 1)).to(dev)
+    actor, critic = mlp(3), mlp(4)
+    at, ct = copy.deepcopy(actor), copy.deepcopy(critic)
+    oa, oc = torch.optim.Adam(actor.parameters(), lr=3e-4), torch.optim.Adam(critic.parameters(), lr=3e-4)
+    C, B = 1 << 20, 256
+    obs, nobs = torch.randn(C, 3, device=dev), torch.randn(C, 3, device=dev)
+    act, rew, term = torch.rand(C, 1, device=dev) * 4 - 2, torch.randn(C, 1, device=dev), torch.zeros(C, 1, device=dev)
+
+    def step(i):
+        idx = torch.randperm(C, device=dev)[:B]
+        o, a, r, n, d = obs[idx], act[idx], rew[idx], nobs[idx], term[idx]
+        with torch.no_grad():
+            y = r + 0.99 * (1 - d) * ct(torch.cat([n, 2 * torch.tanh(at(n))], 1))
+        loss = ((critic(torch.cat([o, a], 1)) - y) ** 2).mean()
+        oc.zero_grad(); loss.backward(); oc.step()
+        if i % 2 == 1:
+            al = -critic(torch.cat([o, 2 * torch.tanh(actor(o))], 1)).mean()
+            oa.zero_grad(); al.backward(); oa.step()
+            with torch.no_grad():
+                for net, tgt in ((actor, at), (critic, ct)):
+                    for p, tp in zip(net.parameters(), tgt.parameters()):
+                        tp.mul_(0.995).add_(0.005 * p)
+
+    for i in range(20):
+        step(i)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for i in range(reps):
+        step(i)
+    torch.cuda.synchronize()
+    return {"eager_us_per_learning_step": (time.perf_counter() - t0) / reps * 1e6}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--iters", type=int, default=2000)
+    ap.add_argument("--out", default=None)
+    ap.add_argument("--trace-dir", default=None, help="write the profiled run's Chrome trace here")
+    args = ap.parse_args()
+    import torch
+    if not torch.cuda.is_available():
+        sys.exit("ddpg_bench needs a GPU")
+    res = {**card()}
+    res["n4096"] = timed(torch, 4096, args.iters)
+    res["n1"] = timed(torch, 1, args.iters * 5)
+    res["profile_n4096"] = profiled(torch, 200, args.trace_dir)
+    res.update(eager(torch))
+    line = json.dumps(res)
+    print(line)
+    if args.out:
+        with open(args.out, "w") as f:
+            f.write(line + "\n")
+
+
+if __name__ == "__main__":
+    main()
