@@ -9,7 +9,7 @@ nothing — the library is dlopen'ed on first use and there is no CPU fallback.
 from . import _abi  # noqa: F401
 from .config import PPOConfig, argparse_struct  # noqa: F401
 
-__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "DDPGConfig", "argparse_struct", "ppo", "a2c", "dqn", "ddpg", "PPOHandle", "Networks", "Logger",
+__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "DDPGConfig", "TD3Config", "argparse_struct", "ppo", "a2c", "dqn", "ddpg", "td3", "PPOHandle", "Networks", "Logger",
            "ConfigParser"]
 
 
@@ -37,7 +37,16 @@ def ddpg(*args, **kwargs):
     return _ddpg(*args, **kwargs)
 
 
+def td3(*args, **kwargs):
+    """Vectorised TD3 on Pendulum (pinned to include/cleanrl_td3.h; the reference has no TD3); see td3_algo.py"""
+    from .td3_algo import td3 as _td3
+    return _td3(*args, **kwargs)
+
+
 def __getattr__(name):
+    if name == "TD3Config":
+        from .td3_algo import TD3Config
+        return TD3Config
     if name == "DDPGConfig":
         from .ddpg_algo import DDPGConfig
         return DDPGConfig

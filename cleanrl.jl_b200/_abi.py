@@ -116,3 +116,23 @@ def make_ddpg_config(num_envs=1, buffer_size=1_000_000, learning_starts=25_000, 
     """crl_ddpg_config with CleanRL's ddpg_continuous_action.py defaults (PendulumEnv() max_steps = 200)."""
     return crl_ddpg_config(C.sizeof(crl_ddpg_config), num_envs, buffer_size, learning_starts, batch_size, train_freq,
                            policy_frequency, max_episode_steps, device, 0, gamma, tau, lr, exploration_noise, seed)
+
+
+# ---- TD3 (include/cleanrl_td3.h) -----------------------------------------------------------------------------
+class crl_td3_config(C.Structure):
+    _fields_ = crl_ddpg_config._fields_ + [("policy_noise", C.c_double), ("noise_clip", C.c_double)]
+
+
+class crl_td3_stats(C.Structure):
+    _fields_ = [("qf1_loss", C.c_double), ("qf2_loss", C.c_double), ("actor_loss", C.c_double), ("sum_return", C.c_double),
+                ("sum_length", C.c_double), ("episodes", C.c_int64), ("learn_steps", C.c_int64), ("actor_steps", C.c_int64),
+                ("iterations", C.c_int64), ("kernel_launches", C.c_int64)]
+
+
+def make_td3_config(num_envs=1, buffer_size=1_000_000, learning_starts=25_000, batch_size=256, train_freq=1, policy_frequency=2,
+                    max_episode_steps=200, device=0, gamma=0.99, tau=0.005, lr=3e-4, exploration_noise=0.1, seed=1,
+                    policy_noise=0.2, noise_clip=0.5):
+    """crl_td3_config with CleanRL's td3_continuous_action.py defaults (PendulumEnv() max_steps = 200)."""
+    return crl_td3_config(C.sizeof(crl_td3_config), num_envs, buffer_size, learning_starts, batch_size, train_freq,
+                          policy_frequency, max_episode_steps, device, 0, gamma, tau, lr, exploration_noise, seed,
+                          policy_noise, noise_clip)

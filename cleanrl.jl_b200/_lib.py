@@ -94,6 +94,19 @@ DDPG_SIGNATURES = {
     "crl_ddpg_actor_loss_raw": (C.c_int, [V, V, I32, V, V, V, V]),
 }
 
+# every symbol include/cleanrl_td3.h declares (the TD3 handle and its raw critic step)
+TD3_SIGNATURES = {
+    "crl_td3_create": (C.c_int, [C.POINTER(_abi.crl_td3_config), C.POINTER(V)]),
+    "crl_td3_destroy": (C.c_int, [V]),
+    "crl_td3_set_params": (C.c_int, [V, V, I32, V, I32, V, I32]),
+    "crl_td3_get_params": (C.c_int, [V] * 7),
+    "crl_td3_get_adam_state": (C.c_int, [V] * 8),
+    "crl_td3_reset": (C.c_int, [V]),
+    "crl_td3_run": (C.c_int, [V, I64, V]),
+    "crl_td3_read_buffer": (C.c_int, [V] * 8),
+    "crl_td3_critic_loss_raw": (C.c_int, [V] * 5 + [I32] + [V] * 5 + [F64, F64, F64, U64, U64] + [V] * 5),
+}
+
 
 def load():
     """dlopen the CUDA library and bind every entry point. Raises if it is not built."""
@@ -104,7 +117,7 @@ def load():
         raise CleanRLCudaError(-2, "%s is not built (run `python cleanrl.jl_b200/build.py` or "
                                    "__graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = C.CDLL(LIB_PATH, mode=C.RTLD_GLOBAL)
-    for name, (res, args) in list(SIGNATURES.items()) + list(DDPG_SIGNATURES.items()):
+    for name, (res, args) in list(SIGNATURES.items()) + list(DDPG_SIGNATURES.items()) + list(TD3_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError here = header/library mismatch
         fn.restype = res
         fn.argtypes = args

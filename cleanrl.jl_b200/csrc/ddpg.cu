@@ -24,6 +24,15 @@
 //   ddpg_update_kernel<IN>  part 2 for either net: one thread per parameter sums its gradient over the batch in ascending
 //                           sample order (deterministic, no float atomics) and applies Adam in place.
 //   ddpg_polyak_kernel      theta' <- tau theta + (1 - tau) theta' for both targets, after the actor step only.
+//
+// TD3 (crl_td3_* of include/cleanrl_td3.h) runs on the same acting kernel, ring, batch sampling, actor step and Polyak
+// kernel; only its critic step is its own:
+//   td3_critic_fwd_kernel     grid (ceil(B/16), 2), blockIdx.y = k picks qf1 or qf2: gather, target actor, clipped
+//                             smoothing noise (Philox stream 7), both target critics, y from their minimum (Float64),
+//                             then critic k's forward, loss and backward into scratch k.
+//   td3_critic_update_kernel  both critics' reductions and Adam steps in one launch (blockIdx.y picks the net); the body
+//                             is ddpg_update_kernel's.
+//   td3_polyak_kernel         qf2' after the actor step; ddpg_polyak_kernel does actor' and qf1'.
 // The raw entry points run the same kernels on rows the caller passes in (sample b = row b), with the gradient written
 // out instead of an Adam step, so that each can be compared with a reference on its own. Every decision that only
 // depends on counters (learn on this iteration?, actor step?, Adam's beta powers) is taken on the host, so a run is a
@@ -35,6 +44,7 @@
 #include <string>
 
 #include "../../include/cleanrl_ddpg.h"
+#include "../../include/cleanrl_td3.h"
 #include "device_math.cuh"
 #include "kernels.h"
 
@@ -52,7 +62,7 @@ using CNet = DNet<DD_D + DD_A>;    // critic Q
 static_assert(ANet::P == CRL_DDPG_ACTOR_PARAMS && CNet::P == CRL_DDPG_CRITIC_PARAMS, "parameter counts");
 static_assert(ANet::W2 % 4 == 0 && CNet::W2 % 4 == 0, "128-bit weight loads of the hidden layer");
 
-constexpr uint32_t STREAM_DDPG_ACT = 5u, STREAM_DDPG_BATCH = 6u;
+constexpr uint32_t STREAM_DDPG_ACT = 5u, STREAM_DDPG_BATCH = 6u, STREAM_TD3_SMOOTH = 7u;
 constexpr int ACT_E = 32;                 // envs per CTA in ddpg_act_kernel
 constexpr int ACT_SP = ACT_E + 4;         // activation row stride (floats): rows stay 16-byte aligned
 constexpr int ACT_T = 256;                // threads of ddpg_act_kernel
@@ -451,12 +461,11 @@ struct UpdArgs {
   double lr, bp1, bp2;     // beta1^t, beta2^t of Adam, kept on the host
 };
 
-// One thread per parameter of a DNet<IN>: its gradient summed over the batch in ascending sample order (one fmaf chain),
-// then Flux.Adam / torch.optim.Adam in the form of dqn_adam: Float64 scalars, Float32 state.
+// Parameter i of a DNet<IN>: its gradient summed over the batch in ascending sample order (one fmaf chain), then
+// Flux.Adam / torch.optim.Adam in the form of dqn_adam: Float64 scalars, Float32 state. Thread 0 also writes the loss.
 template <int IN>
-__global__ void __launch_bounds__(LU_T) ddpg_update_kernel(UpdArgs a) {
+__device__ __forceinline__ void update_param(const UpdArgs& a, int i) {
   using N = DNet<IN>;
-  const int i = blockIdx.x * LU_T + threadIdx.x;
   if (i == 0) {
     double sum = 0.0;
     for (int c = 0; c < a.n_parts; c++) sum += a.loss_part[c];
@@ -493,6 +502,12 @@ __global__ void __launch_bounds__(LU_T) ddpg_update_kernel(UpdArgs a) {
   a.params[i] = __fsub_rn(p0, step);
 }
 
+// one thread per parameter of one net
+template <int IN>
+__global__ void __launch_bounds__(LU_T) ddpg_update_kernel(UpdArgs a) {
+  update_param<IN>(a, blockIdx.x * LU_T + threadIdx.x);
+}
+
 // theta' <- tau theta + (1 - tau) theta' for the actor (i < ANet::P) and the critic, in Float64 and rounded once
 __global__ void __launch_bounds__(256) ddpg_polyak_kernel(const float* actor, float* actor_tgt, const float* critic, float* critic_tgt, double tau) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -500,6 +515,99 @@ __global__ void __launch_bounds__(256) ddpg_polyak_kernel(const float* actor, fl
   float* t = i < ANet::P ? actor_tgt + i : critic_tgt + (i - ANet::P);
   if (i >= ANet::P + CNet::P) return;
   *t = (float)__dadd_rn(__dmul_rn(tau, (double)*p), __dmul_rn(1.0 - tau, (double)*t));
+}
+
+// ---- TD3: twin critics with target-policy smoothing on the DDPG kernels (include/cleanrl_td3.h)
+struct Td3Args {
+  LearnArgs l;                        // actor_tgt, critic = qf1, critic_tgt = qf1', the batch, and qf1's scratch and loss parts
+  const float *critic2, *critic2_tgt; // qf2, qf2'
+  Scratch s2;
+  double* loss_part2;
+  float policy_noise, noise_clip;
+};
+
+// Part 1 of the learning step of both critics, grid (ceil(B/16), 2): blockIdx.y = k picks qf(k+1). Every CTA gathers its
+// 16 samples, runs the target actor, draws the clipped smoothing noise (Philox stream 7, word = position in the batch,
+// counter = learning-step index), runs both target critics, forms y from their minimum with DDPG's expression, and then
+// runs critic k's forward and backward into scratch k. The two y-halves of a sample run the same instructions on the same
+// inputs, so both critics regress on bit-identical targets.
+__global__ void __launch_bounds__(LF_T) td3_critic_fwd_kernel(Td3Args t) {
+  extern __shared__ __align__(16) float smem[];
+  constexpr int SP = LF_SP;
+  const LearnArgs& a = t.l;
+  const int k = blockIdx.y;
+  float* pat = smem;                      // target actor
+  float* pq1t = pat + ANet::PP;           // qf1'
+  float* pq2t = pq1t + CNet::PP;          // qf2'
+  float* pc = pq2t + CNet::PP;            // critic k
+  float* h1 = pc + CNet::PP;              // [64][SP]
+  float* h2 = h1 + DD_H * SP;             // [64][SP]
+  float* z2 = h2 + DD_H * SP;             // [64][SP]
+  float* xin = z2 + DD_H * SP;            // [4][SP] obs, action
+  float* xn = xin + 4 * SP;               // [4][SP] next_obs, smoothed mu'(next_obs)
+  float* out = xn + 4 * SP;               // [SP]
+  float* dout = out + SP;                 // [SP]
+  __shared__ float s_rew[LF_S];
+  __shared__ int s_term[LF_S];
+  const int tid = threadIdx.x, B = a.B, b0 = blockIdx.x * LF_S;
+  float o[DD_D] = {0.0f, 0.0f, 0.0f}, nx[DD_D] = {0.0f, 0.0f, 0.0f}, act = 0.0f, rew = 0.0f;
+  int term = 0;
+  if (tid < LF_S && b0 + tid < B) {
+    const uint32_t idx = batch_row(a, b0 + tid);
+#pragma unroll
+    for (int c = 0; c < DD_D; c++) { o[c] = a.b_obs[idx * DD_D + c]; nx[c] = a.b_next[idx * DD_D + c]; }
+    act = a.b_act[idx]; rew = a.b_rew[idx]; term = a.b_term[idx];
+  }
+  load_params<ANet::P, LF_T>(a.actor_tgt, pat, tid);
+  load_params<CNet::P, LF_T>(a.critic_tgt, pq1t, tid);
+  load_params<CNet::P, LF_T>(t.critic2_tgt, pq2t, tid);
+  load_params<CNet::P, LF_T>(k ? t.critic2 : a.critic, pc, tid);
+  if (tid < LF_S) {
+#pragma unroll
+    for (int c = 0; c < DD_D; c++) { xin[c * SP + tid] = o[c]; xn[c * SP + tid] = nx[c]; }
+    xin[DD_D * SP + tid] = act;
+    s_rew[tid] = rew; s_term[tid] = term;
+  }
+  __syncthreads();
+  mlp_forward<DD_D, LF_S, SP, LF_T>(pat, xn, h1, h2, out, tid);             // target_actor(next_obs)
+  if (tid < LF_S) {
+    // eps = clamp(policy_noise z, -noise_clip, noise_clip) * 2 with z Box-Muller as in ddpg_act_kernel; every operation
+    // in Float32 in this order (no contraction), then a' = clamp(mu' + eps, -2, 2)
+    uint32_t r[4];
+    philox_draw(a.seed, (uint32_t)(b0 + tid), a.learn_step, STREAM_TD3_SMOOTH, r);
+    const float u1 = (float)((r[0] >> 8) + 1u) * (1.0f / 16777216.0f);
+    const float u2 = (float)(r[1] >> 8) * (1.0f / 16777216.0f);
+    const float z = sqrtf(-2.0f * logf(u1)) * cosf(6.283185307179586f * u2);
+    const float eps = __fmul_rn(fminf(fmaxf(__fmul_rn(t.policy_noise, z), -t.noise_clip), t.noise_clip), DD_MAX_TORQUE);
+    xn[DD_D * SP + tid] = fminf(fmaxf(__fadd_rn(actor_out(out[tid]), eps), -DD_MAX_TORQUE), DD_MAX_TORQUE);
+  }
+  __syncthreads();
+  mlp_forward<DD_D + DD_A, LF_S, SP, LF_T>(pq1t, xn, h1, h2, out, tid);     // qf1_target(next_obs, a')
+  const float q1n = tid < LF_S ? out[tid] : 0.0f;
+  mlp_forward<DD_D + DD_A, LF_S, SP, LF_T>(pq2t, xn, h1, h2, out, tid);     // qf2_target(next_obs, a')
+  double y = 0.0;
+  if (tid < LF_S) y = (double)s_rew[tid] + a.gamma * (1.0 - (double)s_term[tid]) * (double)fminf(q1n, out[tid]);
+  mlp_forward<DD_D + DD_A, LF_S, SP, LF_T>(pc, xin, h1, h2, out, tid);      // qf_k(obs, action)
+  if (tid < LF_S) {
+    const bool in = b0 + tid < B;
+    const double diff = (double)out[tid] - y;
+    dout[tid] = in ? (float)(2.0 * diff / (double)B) : 0.0f;               // d mse / d q
+    block_part(in ? diff * diff : 0.0, k ? t.loss_part2 : a.loss_part);
+  }
+  __syncthreads();
+  mlp_backward<DD_D + DD_A, LF_S, SP, LF_T>(pc, xin, h1, h2, dout, z2, nullptr, k ? t.s2 : a.s, b0, B, true, tid);
+}
+
+// part 2 of both critics in one launch: blockIdx.y picks the net, its scratch, its loss parts and its Adam state
+__global__ void __launch_bounds__(LU_T) td3_critic_update_kernel(UpdArgs q1, UpdArgs q2) {
+  update_param<DD_D + DD_A>(blockIdx.y ? q2 : q1, blockIdx.x * LU_T + threadIdx.x);
+}
+
+// qf2' <- tau qf2 + (1 - tau) qf2', as ddpg_polyak_kernel does for the actor and qf1
+__global__ void __launch_bounds__(256) td3_polyak_kernel(const float* critic2, float* critic2_tgt, double tau) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= CNet::P) return;
+  critic2_tgt[i] = (float)__dadd_rn(__dmul_rn(tau, (double)critic2[i]), __dmul_rn(1.0 - tau, (double)critic2_tgt[i]));
 }
 
 __global__ void ddpg_reset_kernel(int N, unsigned long long seed, float* env_state, int* env_t, double* ep_ret, int* ep_len, uint32_t* resets) {
@@ -517,7 +625,9 @@ constexpr size_t ACT_SMEM = (ANet::PP + (2 * DD_H + 1 + DD_D) * ACT_SP) * sizeof
 constexpr size_t FWD_RAW_SMEM = (ANet::PP + CNet::PP + (2 * DD_H + 1 + 4) * ACT_SP) * sizeof(float);
 constexpr size_t CF_SMEM = (ANet::PP + 2 * CNet::PP + (3 * DD_H + 8 + 2) * LF_SP) * sizeof(float);
 constexpr size_t AF_SMEM = (ANet::PP + CNet::PP + (6 * DD_H + 4 + 2) * LF_SP) * sizeof(float);
+constexpr size_t TCF_SMEM = (ANet::PP + 3 * CNet::PP + (3 * DD_H + 8 + 2) * LF_SP) * sizeof(float);
 static_assert(ACT_SMEM <= 227 * 1024 && FWD_RAW_SMEM <= 227 * 1024 && CF_SMEM <= 227 * 1024 && AF_SMEM <= 227 * 1024, "ddpg shared memory");
+static_assert(TCF_SMEM <= 227 * 1024, "td3 shared memory");
 constexpr size_t SCRATCH_FLOATS = (size_t)LEARN_B * (XS + 4 * DD_H + 1);
 
 int dfail(int code, const std::string& msg) { return crl_internal_fail(code, msg.c_str()); }
@@ -546,6 +656,7 @@ cudaError_t set_smem_attrs() {
   if (e == cudaSuccess) e = cudaFuncSetAttribute(ddpg_forward_raw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FWD_RAW_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(ddpg_critic_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CF_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(ddpg_actor_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AF_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(td3_critic_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TCF_SMEM);
   return e;
 }
 
@@ -559,6 +670,19 @@ cudaError_t launch_net_step(bool critic, const LearnArgs& l, UpdArgs u, cudaStre
   u.s = l.s; u.loss_part = l.loss_part; u.n_parts = fwd_blocks; u.B = l.B; u.loss_sign = critic ? 1.0 : -1.0;
   if (critic) ddpg_update_kernel<DD_D + DD_A><<<(CNet::P + LU_T - 1) / LU_T, LU_T, 0, s>>>(u);
   else ddpg_update_kernel<DD_D><<<(ANet::P + LU_T - 1) / LU_T, LU_T, 0, s>>>(u);
+  return cudaGetLastError();
+}
+
+// TD3's critic step: both critics' forward + deltas in one launch, then both reductions with Adam (or without) in one
+cudaError_t launch_td3_critic_step(const Td3Args& t, UpdArgs u1, UpdArgs u2, cudaStream_t s) {
+  const int fwd_blocks = (t.l.B + LF_S - 1) / LF_S;
+  td3_critic_fwd_kernel<<<dim3(fwd_blocks, 2), LF_T, TCF_SMEM, s>>>(t);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  u1.s = t.l.s; u1.loss_part = t.l.loss_part;
+  u2.s = t.s2; u2.loss_part = t.loss_part2;
+  for (UpdArgs* u : {&u1, &u2}) { u->n_parts = fwd_blocks; u->B = t.l.B; u->loss_sign = 1.0; }
+  td3_critic_update_kernel<<<dim3((CNet::P + LU_T - 1) / LU_T, 2), LU_T, 0, s>>>(u1, u2);
   return cudaGetLastError();
 }
 
@@ -700,65 +824,86 @@ extern "C" CRL_API int crl_ddpg_reset(crl_ddpg_ctx* c) {
   return CRL_OK;
 }
 
+// One acting launch for every iteration from k up to (and including) the next learning step: the parameters are constant
+// in between. Bounded by `iterations`, by ACT_MAX_STEPS and by the ring capacity (steps of one launch must not share a
+// slot). Advances k and the iteration, ring and launch counters; `learn` is set when the last iteration learns.
+static int act_launch(crl_ddpg_ctx* c, int64_t iterations, int64_t& k, bool& learn) {
+  const crl_ddpg_config& g = c->cfg;
+  const int N = g.num_envs, C = g.buffer_size;
+  ActArgs a;
+  a.actor = c->actor; a.env_state = c->env_state; a.env_t = c->env_t; a.ep_ret = c->ep_ret; a.ep_len = c->ep_len; a.resets = c->resets;
+  a.b_obs = c->b_obs; a.b_next = c->b_next; a.b_act = c->b_act; a.b_rew = c->b_rew; a.b_term = c->b_term; a.dev = c->dev;
+  a.seed = g.seed; a.it0 = (unsigned long long)(c->it + 1); a.learning_starts = g.learning_starts;
+  a.sigma = (float)(g.exploration_noise * (double)DD_MAX_TORQUE);
+  a.N = N; a.C = C; a.ptr = c->ptr; a.max_steps = g.max_episode_steps;
+  int ns = 0;
+  learn = false;
+  while (k < iterations && ns < ACT_MAX_STEPS && (long long)(ns + 1) * N <= (long long)C && !learn) {
+    c->it += 1;
+    k += 1;
+    ns += 1;
+    c->ptr = (int)(((long long)c->ptr + N) % C);
+    c->size = c->size + N > C ? C : c->size + N;
+    const long long gs = c->it * (long long)N;
+    learn = gs > (long long)g.learning_starts && c->it % g.train_freq == 0 && c->size >= g.batch_size;
+  }
+  a.n_steps = ns;
+  ddpg_act_kernel<<<(N + ACT_E - 1) / ACT_E, ACT_T, ACT_SMEM, c->stream>>>(a);
+  DCK(cudaGetLastError());
+  c->launches += 1;
+  return CRL_OK;
+}
+
+// the learning step's batch: Philox stream 6 keyed by the learning-step index, over the ring's current size
+static LearnArgs learn_args(const crl_ddpg_ctx* c, const Scratch& s) {
+  LearnArgs l;
+  memset(&l, 0, sizeof(l));
+  l.actor = c->actor; l.critic = c->critic; l.actor_tgt = c->actor_tgt; l.critic_tgt = c->critic_tgt;
+  l.b_obs = c->b_obs; l.b_next = c->b_next; l.b_act = c->b_act; l.b_rew = c->b_rew; l.b_term = c->b_term;
+  l.seed = c->cfg.seed; l.learn_step = (unsigned long long)c->learn_steps; l.gamma = c->cfg.gamma; l.B = c->cfg.batch_size;
+  l.size = c->size; l.s = s; l.loss_part = c->loss_part;
+  return l;
+}
+
+// every policy_frequency-th learning step, on the same batch and against the critic just updated: the actor's step,
+// then Polyak averaging of the actor's and the critic's targets
+static int actor_step(crl_ddpg_ctx* c, const LearnArgs& l) {
+  UpdArgs u;
+  memset(&u, 0, sizeof(u));
+  u.params = c->actor; u.m = c->am; u.v = c->av; u.loss_out = &c->dev->actor_loss; u.lr = c->cfg.lr; u.bp1 = c->abp1; u.bp2 = c->abp2;
+  DCK(launch_net_step(false, l, u, c->stream));
+  ddpg_polyak_kernel<<<(ANet::P + CNet::P + 255) / 256, 256, 0, c->stream>>>(c->actor, c->actor_tgt, c->critic, c->critic_tgt, c->cfg.tau);
+  DCK(cudaGetLastError());
+  c->abp1 *= 0.9; c->abp2 *= 0.999;
+  c->launches += 3;
+  c->actor_steps += 1;
+  return CRL_OK;
+}
+
 extern "C" CRL_API int crl_ddpg_run(crl_ddpg_ctx* c, int64_t iterations, crl_ddpg_stats* stats) {
   if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
   if (iterations < 0) return dfail(CRL_ERR_INVALID, "iterations must be >= 0");
   if (!c->params_set) return dfail(CRL_ERR_STATE, "crl_ddpg_run called before crl_ddpg_set_params");
   if (!c->reset_done) return dfail(CRL_ERR_STATE, "crl_ddpg_run called before crl_ddpg_reset");
   DCK(cudaSetDevice(c->cfg.device));
-  const crl_ddpg_config& g = c->cfg;
-  const int N = g.num_envs, C = g.buffer_size;
   // per-call episode aggregate: clear the three accumulators, keep the last losses
   DCK(cudaMemsetAsync(&c->dev->sum_return, 0, sizeof(double) * 2 + sizeof(unsigned long long), c->stream));
   const Scratch s = carve(c->scratch);
   int64_t k = 0;
   while (k < iterations) {
-    // One launch acts for every iteration up to (and including) the next learning step: the parameters are constant in
-    // between. Bounded by ACT_MAX_STEPS and by the ring capacity (steps of one launch must not share a slot).
-    ActArgs a;
-    a.actor = c->actor; a.env_state = c->env_state; a.env_t = c->env_t; a.ep_ret = c->ep_ret; a.ep_len = c->ep_len; a.resets = c->resets;
-    a.b_obs = c->b_obs; a.b_next = c->b_next; a.b_act = c->b_act; a.b_rew = c->b_rew; a.b_term = c->b_term; a.dev = c->dev;
-    a.seed = g.seed; a.it0 = (unsigned long long)(c->it + 1); a.learning_starts = g.learning_starts;
-    a.sigma = (float)(g.exploration_noise * (double)DD_MAX_TORQUE);
-    a.N = N; a.C = C; a.ptr = c->ptr; a.max_steps = g.max_episode_steps;
-    int ns = 0;
     bool learn = false;
-    while (k < iterations && ns < ACT_MAX_STEPS && (long long)(ns + 1) * N <= (long long)C && !learn) {
-      c->it += 1;
-      k += 1;
-      ns += 1;
-      c->ptr = (int)(((long long)c->ptr + N) % C);
-      c->size = c->size + N > C ? C : c->size + N;
-      const long long gs = c->it * (long long)N;
-      learn = gs > (long long)g.learning_starts && c->it % g.train_freq == 0 && c->size >= g.batch_size;
-    }
-    a.n_steps = ns;
-    ddpg_act_kernel<<<(N + ACT_E - 1) / ACT_E, ACT_T, ACT_SMEM, c->stream>>>(a);
-    DCK(cudaGetLastError());
-    c->launches += 1;
+    if (int rc = act_launch(c, iterations, k, learn)) return rc;
     if (!learn) continue;
-    LearnArgs l;
-    memset(&l, 0, sizeof(l));
-    l.actor = c->actor; l.critic = c->critic; l.actor_tgt = c->actor_tgt; l.critic_tgt = c->critic_tgt;
-    l.b_obs = c->b_obs; l.b_next = c->b_next; l.b_act = c->b_act; l.b_rew = c->b_rew; l.b_term = c->b_term;
-    l.seed = g.seed; l.learn_step = (unsigned long long)c->learn_steps; l.gamma = g.gamma; l.B = g.batch_size; l.size = c->size;
-    l.s = s; l.loss_part = c->loss_part;
+    const LearnArgs l = learn_args(c, s);
     UpdArgs u;
     memset(&u, 0, sizeof(u));
-    u.params = c->critic; u.m = c->cm; u.v = c->cv; u.loss_out = &c->dev->critic_loss; u.lr = g.lr; u.bp1 = c->cbp1; u.bp2 = c->cbp2;
+    u.params = c->critic; u.m = c->cm; u.v = c->cv; u.loss_out = &c->dev->critic_loss; u.lr = c->cfg.lr; u.bp1 = c->cbp1; u.bp2 = c->cbp2;
     DCK(launch_net_step(true, l, u, c->stream));
     c->cbp1 *= 0.9; c->cbp2 *= 0.999;
     c->launches += 2;
     c->learn_steps += 1;
-    if (c->learn_steps % g.policy_frequency == 0) {   // every policy_frequency-th learning step, against the updated critic
-      u.params = c->actor; u.m = c->am; u.v = c->av; u.loss_out = &c->dev->actor_loss; u.bp1 = c->abp1; u.bp2 = c->abp2;
-      DCK(launch_net_step(false, l, u, c->stream));
-      ddpg_polyak_kernel<<<(ANet::P + CNet::P + 255) / 256, 256, 0, c->stream>>>(c->actor, c->actor_tgt, c->critic, c->critic_tgt, g.tau);
-      DCK(cudaGetLastError());
-      c->abp1 *= 0.9; c->abp2 *= 0.999;
-      c->launches += 3;
-      c->actor_steps += 1;
-    }
+    if (c->learn_steps % c->cfg.policy_frequency == 0)
+      if (int rc = actor_step(c, l)) return rc;
   }
   if (stats) {
     DdpgDev d;
@@ -854,4 +999,214 @@ extern "C" CRL_API int crl_ddpg_actor_loss_raw(const float* actor, const float* 
   memset(&l, 0, sizeof(l));
   l.actor = actor; l.critic = critic; l.b_obs = obs; l.B = B;
   return ddpg_loss_raw(false, l, grads_out, loss_out, (cudaStream_t)stream);
+}
+
+// ---- TD3 (include/cleanrl_td3.h). The DDPG context carries everything the two share: envs, ring, actor, qf1 (as the
+// critic), the actor's and qf1's targets, their Adam state and the counters. Both critics share one step count, so
+// qf2's Adam uses the critic's beta powers.
+struct crl_td3_ctx {
+  crl_ddpg_ctx* d;
+  crl_td3_config cfg;
+  float *critic2, *critic2_tgt, *c2m, *c2v;
+  float* scratch2;
+  double *loss_part2, *qf2_loss;
+};
+
+static crl_ddpg_config td3_ddpg_config(const crl_td3_config& t) {
+  crl_ddpg_config g;
+  memset(&g, 0, sizeof(g));
+  g.struct_size = (int32_t)sizeof(crl_ddpg_config);
+  g.num_envs = t.num_envs; g.buffer_size = t.buffer_size; g.learning_starts = t.learning_starts; g.batch_size = t.batch_size;
+  g.train_freq = t.train_freq; g.policy_frequency = t.policy_frequency; g.max_episode_steps = t.max_episode_steps;
+  g.device = t.device; g.gamma = t.gamma; g.tau = t.tau; g.lr = t.lr; g.exploration_noise = t.exploration_noise; g.seed = t.seed;
+  return g;
+}
+
+static int td3_validate_noise(double policy_noise, double noise_clip) {
+  if (!(policy_noise >= 0.0 && isfinite(policy_noise)) || !(noise_clip >= 0.0 && isfinite(noise_clip)))
+    return dfail(CRL_ERR_INVALID, "policy_noise and noise_clip must be finite and >= 0");
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_td3_destroy(crl_td3_ctx* c) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  if (c->d) {
+    cudaSetDevice(c->cfg.device);
+    cudaStreamSynchronize(c->d->stream);
+  }
+  void* ptrs[] = {c->critic2, c->critic2_tgt, c->c2m, c->c2v, c->scratch2, c->loss_part2, c->qf2_loss};
+  for (void* p : ptrs) if (p) cudaFree(p);
+  if (c->d) crl_ddpg_destroy(c->d);
+  delete c;
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_td3_create(const crl_td3_config* cfg, crl_td3_ctx** out) {
+  if (!cfg || !out) return dfail(CRL_ERR_INVALID, "NULL argument");
+  *out = nullptr;
+  if (cfg->struct_size != (int32_t)sizeof(crl_td3_config)) return dfail(CRL_ERR_INVALID, "crl_td3_config.struct_size mismatch");
+  if (int rc = td3_validate_noise(cfg->policy_noise, cfg->noise_clip)) return rc;
+  const crl_ddpg_config g = td3_ddpg_config(*cfg);
+  if (int rc = ddpg_validate(&g)) return rc;
+  crl_ddpg_ctx* d = nullptr;
+  if (int rc = crl_ddpg_create(&g, &d)) return rc;   // checks the device, then allocates
+  crl_td3_ctx* c = new crl_td3_ctx();
+  memset(c, 0, sizeof(*c));
+  c->d = d;
+  c->cfg = *cfg;
+#define TCKC(call)                                                                                            \
+  do {                                                                                                        \
+    cudaError_t e__ = (call);                                                                                 \
+    if (e__ != cudaSuccess) {                                                                                 \
+      crl_td3_destroy(c);                                                                                     \
+      return dfail(CRL_ERR_CUDA, std::string(#call) + " failed: " + cudaGetErrorString(e__) + " (ddpg.cu)"); \
+    }                                                                                                         \
+  } while (0)
+  TCKC(dzalloc(&c->critic2, CNet::PP)); TCKC(dzalloc(&c->critic2_tgt, CNet::PP)); TCKC(dzalloc(&c->c2m, CNet::P));
+  TCKC(dzalloc(&c->c2v, CNet::P)); TCKC(dzalloc(&c->scratch2, SCRATCH_FLOATS)); TCKC(dzalloc(&c->loss_part2, LF_MAX_BLOCKS));
+  TCKC(dzalloc(&c->qf2_loss, 1));
+#undef TCKC
+  *out = c;
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_td3_set_params(crl_td3_ctx* c, const float* actor, int32_t n_actor, const float* qf1, int32_t n_qf1,
+                                          const float* qf2, int32_t n_qf2) {
+  if (!c || !actor || !qf1 || !qf2) return dfail(CRL_ERR_INVALID, "NULL argument");
+  if (n_actor != ANet::P || n_qf1 != CNet::P || n_qf2 != CNet::P)
+    return dfail(CRL_ERR_INVALID, "TD3 parameter vectors must have 4481 (actor) and 4545 (qf1, qf2) floats");
+  if (int rc = crl_ddpg_set_params(c->d, actor, n_actor, qf1, n_qf1)) return rc;
+  c->d->params_set = false;   // until qf2 is in place as well
+  const cudaStream_t s = c->d->stream;
+  DCK(cudaMemcpyAsync(c->critic2, qf2, sizeof(float) * CNet::P, cudaMemcpyHostToDevice, s));
+  DCK(cudaMemcpyAsync(c->critic2_tgt, c->critic2, sizeof(float) * CNet::P, cudaMemcpyDeviceToDevice, s));
+  DCK(cudaMemsetAsync(c->c2m, 0, sizeof(float) * CNet::P, s)); DCK(cudaMemsetAsync(c->c2v, 0, sizeof(float) * CNet::P, s));
+  DCK(cudaMemsetAsync(c->qf2_loss, 0, sizeof(double), s));
+  DCK(cudaStreamSynchronize(s));
+  c->d->params_set = true;
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_td3_get_params(crl_td3_ctx* c, float* actor, float* qf1, float* qf2, float* actor_target, float* qf1_target,
+                                          float* qf2_target) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  if (int rc = crl_ddpg_get_params(c->d, actor, qf1, actor_target, qf1_target)) return rc;
+  if (qf2) DCK(cudaMemcpyAsync(qf2, c->critic2, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->d->stream));
+  if (qf2_target) DCK(cudaMemcpyAsync(qf2_target, c->critic2_tgt, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->d->stream));
+  DCK(cudaStreamSynchronize(c->d->stream));
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_td3_get_adam_state(crl_td3_ctx* c, float* actor_m, float* actor_v, float* qf1_m, float* qf1_v, float* qf2_m,
+                                              float* qf2_v, double* beta_pow) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  if (int rc = crl_ddpg_get_adam_state(c->d, actor_m, actor_v, qf1_m, qf1_v, beta_pow)) return rc;
+  if (qf2_m) DCK(cudaMemcpyAsync(qf2_m, c->c2m, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->d->stream));
+  if (qf2_v) DCK(cudaMemcpyAsync(qf2_v, c->c2v, sizeof(float) * CNet::P, cudaMemcpyDeviceToHost, c->d->stream));
+  DCK(cudaStreamSynchronize(c->d->stream));
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_td3_reset(crl_td3_ctx* c) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  return crl_ddpg_reset(c->d);
+}
+
+extern "C" CRL_API int crl_td3_run(crl_td3_ctx* t, int64_t iterations, crl_td3_stats* stats) {
+  if (!t) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  if (iterations < 0) return dfail(CRL_ERR_INVALID, "iterations must be >= 0");
+  crl_ddpg_ctx* c = t->d;
+  if (!c->params_set) return dfail(CRL_ERR_STATE, "crl_td3_run called before crl_td3_set_params");
+  if (!c->reset_done) return dfail(CRL_ERR_STATE, "crl_td3_run called before crl_td3_reset");
+  DCK(cudaSetDevice(c->cfg.device));
+  DCK(cudaMemsetAsync(&c->dev->sum_return, 0, sizeof(double) * 2 + sizeof(unsigned long long), c->stream));
+  const Scratch s1 = carve(c->scratch), s2 = carve(t->scratch2);
+  int64_t k = 0;
+  while (k < iterations) {
+    bool learn = false;
+    if (int rc = act_launch(c, iterations, k, learn)) return rc;
+    if (!learn) continue;
+    Td3Args a;
+    memset(&a, 0, sizeof(a));
+    a.l = learn_args(c, s1);
+    a.critic2 = t->critic2; a.critic2_tgt = t->critic2_tgt; a.s2 = s2; a.loss_part2 = t->loss_part2;
+    a.policy_noise = (float)t->cfg.policy_noise; a.noise_clip = (float)t->cfg.noise_clip;
+    UpdArgs u1, u2;
+    memset(&u1, 0, sizeof(u1));
+    u1.lr = c->cfg.lr; u1.bp1 = c->cbp1; u1.bp2 = c->cbp2;
+    u2 = u1;
+    u1.params = c->critic; u1.m = c->cm; u1.v = c->cv; u1.loss_out = &c->dev->critic_loss;
+    u2.params = t->critic2; u2.m = t->c2m; u2.v = t->c2v; u2.loss_out = t->qf2_loss;
+    DCK(launch_td3_critic_step(a, u1, u2, c->stream));
+    c->cbp1 *= 0.9; c->cbp2 *= 0.999;
+    c->launches += 2;
+    c->learn_steps += 1;
+    if (c->learn_steps % c->cfg.policy_frequency == 0) {
+      if (int rc = actor_step(c, a.l)) return rc;   // actor against qf1, Polyak of actor' and qf1'
+      td3_polyak_kernel<<<(CNet::P + 255) / 256, 256, 0, c->stream>>>(t->critic2, t->critic2_tgt, c->cfg.tau);
+      DCK(cudaGetLastError());
+      c->launches += 1;
+    }
+  }
+  if (stats) {
+    DdpgDev d;
+    double q2 = 0.0;
+    DCK(cudaMemcpyAsync(&d, c->dev, sizeof(d), cudaMemcpyDeviceToHost, c->stream));
+    DCK(cudaMemcpyAsync(&q2, t->qf2_loss, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    DCK(cudaStreamSynchronize(c->stream));
+    stats->qf1_loss = d.critic_loss; stats->qf2_loss = q2; stats->actor_loss = d.actor_loss; stats->sum_return = d.sum_return;
+    stats->sum_length = d.sum_length; stats->episodes = (int64_t)d.episodes; stats->learn_steps = c->learn_steps;
+    stats->actor_steps = c->actor_steps; stats->iterations = c->it; stats->kernel_launches = c->launches;
+  }
+  return CRL_OK;
+}
+
+extern "C" CRL_API int crl_td3_read_buffer(crl_td3_ctx* c, float* obs, float* action, float* reward, float* next_obs, uint8_t* terminal,
+                                           int32_t* size, int32_t* ptr) {
+  if (!c) return dfail(CRL_ERR_INVALID, "ctx is NULL");
+  return crl_ddpg_read_buffer(c->d, obs, action, reward, next_obs, terminal, size, ptr);
+}
+
+extern "C" CRL_API int crl_td3_critic_loss_raw(const float* actor_target, const float* qf1, const float* qf2, const float* qf1_target,
+                                               const float* qf2_target, int32_t B, const float* obs, const float* action,
+                                               const float* reward, const float* next_obs, const uint8_t* terminal, double gamma,
+                                               double policy_noise, double noise_clip, uint64_t seed, uint64_t learn_step,
+                                               float* qf1_grads_out, float* qf2_grads_out, double* qf1_loss_out,
+                                               double* qf2_loss_out, void* stream) {
+  if (!actor_target || !qf1 || !qf2 || !qf1_target || !qf2_target || !obs || !action || !reward || !next_obs || !terminal ||
+      !qf1_grads_out || !qf2_grads_out || !qf1_loss_out || !qf2_loss_out)
+    return dfail(CRL_ERR_INVALID, "NULL argument");
+  if (((uintptr_t)actor_target | (uintptr_t)qf1 | (uintptr_t)qf2 | (uintptr_t)qf1_target | (uintptr_t)qf2_target) % 16)
+    return dfail(CRL_ERR_INVALID, "parameter vectors must be 16-byte aligned");
+  if (B < 1 || B > LEARN_B) return dfail(CRL_ERR_INVALID, "B must be in [1, 256]");
+  if (int rc = td3_validate_noise(policy_noise, noise_clip)) return rc;
+  if (int rc = ddpg_raw_device_check()) return rc;
+  float* scratch = nullptr;
+  double* dscratch = nullptr;
+  DCK(cudaMalloc(reinterpret_cast<void**>(&scratch), 2 * SCRATCH_FLOATS * sizeof(float)));
+  if (cudaMalloc(reinterpret_cast<void**>(&dscratch), 2 * LF_MAX_BLOCKS * sizeof(double)) != cudaSuccess) {
+    cudaFree(scratch);
+    return dfail(CRL_ERR_CUDA, "cudaMalloc failed (crl_td3_critic_loss_raw)");
+  }
+  Td3Args a;
+  memset(&a, 0, sizeof(a));
+  LearnArgs& l = a.l;
+  l.actor_tgt = actor_target; l.critic = qf1; l.critic_tgt = qf1_target;
+  l.b_obs = obs; l.b_act = action; l.b_rew = reward; l.b_next = next_obs; l.b_term = terminal;
+  l.seed = seed; l.learn_step = learn_step; l.gamma = gamma; l.B = B; l.size = B; l.in_order = 1;
+  l.s = carve(scratch); l.loss_part = dscratch;
+  a.critic2 = qf2; a.critic2_tgt = qf2_target; a.s2 = carve(scratch + SCRATCH_FLOATS); a.loss_part2 = dscratch + LF_MAX_BLOCKS;
+  a.policy_noise = (float)policy_noise; a.noise_clip = (float)noise_clip;
+  UpdArgs u1, u2;
+  memset(&u1, 0, sizeof(u1));
+  u2 = u1;
+  u1.grads_out = qf1_grads_out; u1.loss_out = qf1_loss_out;
+  u2.grads_out = qf2_grads_out; u2.loss_out = qf2_loss_out;
+  const cudaStream_t s = (cudaStream_t)stream;
+  cudaError_t e = launch_td3_critic_step(a, u1, u2, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);   // the scratch is freed below
+  cudaFree(scratch);
+  cudaFree(dscratch);
+  if (e != cudaSuccess) return dfail(CRL_ERR_CUDA, std::string("crl_td3_critic_loss_raw failed: ") + cudaGetErrorString(e));
+  return CRL_OK;
 }

@@ -1,4 +1,4 @@
-"""Time crl_ddpg_run on one GPU and print one JSON line.
+"""Time crl_ddpg_run (or, with --algo td3, crl_td3_run) on one GPU and print one JSON line.
 
 Workload: 4,096 Pendulum envs, a 1,048,576-transition ring, batch 256, a learning step every iteration,
 policy_frequency 2, learning_starts 10,000; and the same with num_envs 1 (one learning step per env step, CleanRL's
@@ -9,7 +9,10 @@ update-to-data ratio). Reported:
     of torch.profiler in a separate profiled run;
   * the same learning step written in PyTorch eager on the same GPU at B = 256, for comparison;
   * the card's name, power limit and max SM clock, read in the same call.
-Usage: python tools/ddpg_bench.py [--iters 2000] [--out path.json]"""
+TD3 runs the same workload with CleanRL's smoothing noise (0.2, clip 0.5); its learning step is the twin-critic pair
+every step and the actor pair + two Polyak launches on every second step. The kernel filter counts the reused ddpg_*
+kernels as well as the td3_* ones.
+Usage: python tools/ddpg_bench.py [--algo {ddpg,td3}] [--iters 2000] [--out path.json]"""
 import argparse
 import json
 import os
@@ -27,19 +30,23 @@ def card():
     return {"gpu": name, "power_limit": power, "max_sm_clock": clock}
 
 
-def make(num_envs):
+def make(num_envs, algo="ddpg"):
     from cleanrl_jl_b200 import _abi
-    from cleanrl_jl_b200.ddpg_algo import DDPGHandle, init_ddpg_params
-    cfg = _abi.make_ddpg_config(num_envs=num_envs, buffer_size=1 << 20, learning_starts=10_000, batch_size=256, train_freq=1,
-                                policy_frequency=2, seed=1)
-    h = DDPGHandle(cfg)
-    h.set_params(*init_ddpg_params(1))
+    kw = dict(num_envs=num_envs, buffer_size=1 << 20, learning_starts=10_000, batch_size=256, train_freq=1, policy_frequency=2, seed=1)
+    if algo == "td3":
+        from cleanrl_jl_b200.td3_algo import TD3Handle, init_td3_params
+        h = TD3Handle(_abi.make_td3_config(**kw))
+        h.set_params(*init_td3_params(1))
+    else:
+        from cleanrl_jl_b200.ddpg_algo import DDPGHandle, init_ddpg_params
+        h = DDPGHandle(_abi.make_ddpg_config(**kw))
+        h.set_params(*init_ddpg_params(1))
     h.reset()
     return h
 
 
-def timed(torch, num_envs, iters):
-    h = make(num_envs)
+def timed(torch, num_envs, iters, algo="ddpg"):
+    h = make(num_envs, algo)
     h.run(10_000 // num_envs + 64)            # warm-up: past learning_starts, every kernel launched
     torch.cuda.synchronize()
     st0 = h.run(0)
@@ -52,10 +59,10 @@ def timed(torch, num_envs, iters):
             "learner_steps_per_s": (st.learn_steps - st0.learn_steps) / dt}
 
 
-def profiled(torch, iters, out_dir):
+def profiled(torch, iters, out_dir, algo="ddpg"):
     """per-kernel device time from torch.profiler (CUDA activities) in a run of its own"""
     from torch.profiler import ProfilerActivity, profile
-    h = make(4096)
+    h = make(4096, algo)
     h.run(10_000 // 4096 + 8)
     torch.cuda.synchronize()
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
@@ -66,27 +73,33 @@ def profiled(torch, iters, out_dir):
     h.close()
     per = {}
     for e in prof.key_averages():
-        if "ddpg" in e.key:
+        if "ddpg" in e.key or "td3" in e.key:
             k = e.key.replace("void ", "").replace("(anonymous namespace)::", "").split("(")[0]
             per[k] = per.get(k, 0.0) + e.device_time_total
     act = sum(v for k, v in per.items() if "act_kernel" in k)
     lrn = sum(v for k, v in per.items() if "act_kernel" not in k)
     if out_dir:
         os.makedirs(out_dir, exist_ok=True)
-        prof.export_chrome_trace(os.path.join(out_dir, "ddpg_trace.json"))
+        prof.export_chrome_trace(os.path.join(out_dir, "%s_trace.json" % algo))
     return {"us_per_acting_launch": act / iters, "us_per_learning_step": lrn / max(learn, 1),
             "kernel_us_total": {k: round(v, 1) for k, v in per.items()}}
 
 
-def eager(torch, reps=200):
-    """the same learning step (critic step every time, actor step + Polyak every second) in PyTorch eager, B = 256"""
+def eager(torch, reps=200, algo="ddpg"):
+    """the same learning step (critic step every time, actor step + Polyak every second) in PyTorch eager, B = 256; TD3:
+    two critics with one Adam over both, the smoothed target action and the minimum of the two target critics"""
     import copy
     nn = torch.nn
     dev = "cuda"
     mlp = lambda i: nn.Sequential(nn.Linear(i, 64), nn.ReLU(), nn.Linear(64, 64), nn.ReLU(), nn.Linear(64, 1)).to(dev)
     actor, critic = mlp(3), mlp(4)
     at, ct = copy.deepcopy(actor), copy.deepcopy(critic)
-    oa, oc = torch.optim.Adam(actor.parameters(), lr=3e-4), torch.optim.Adam(critic.parameters(), lr=3e-4)
+    critic_params = list(critic.parameters())
+    if algo == "td3":
+        critic2 = mlp(4)
+        ct2 = copy.deepcopy(critic2)
+        critic_params += list(critic2.parameters())
+    oa, oc = torch.optim.Adam(actor.parameters(), lr=3e-4), torch.optim.Adam(critic_params, lr=3e-4)
     C, B = 1 << 20, 256
     obs, nobs = torch.randn(C, 3, device=dev), torch.randn(C, 3, device=dev)
     act, rew, term = torch.rand(C, 1, device=dev) * 4 - 2, torch.randn(C, 1, device=dev), torch.zeros(C, 1, device=dev)
@@ -95,14 +108,20 @@ def eager(torch, reps=200):
         idx = torch.randperm(C, device=dev)[:B]
         o, a, r, n, d = obs[idx], act[idx], rew[idx], nobs[idx], term[idx]
         with torch.no_grad():
-            y = r + 0.99 * (1 - d) * ct(torch.cat([n, 2 * torch.tanh(at(n))], 1))
+            if algo == "td3":
+                na = (2 * torch.tanh(at(n)) + (torch.randn_like(a) * 0.2).clamp(-0.5, 0.5) * 2).clamp(-2, 2)
+                y = r + 0.99 * (1 - d) * torch.min(ct(torch.cat([n, na], 1)), ct2(torch.cat([n, na], 1)))
+            else:
+                y = r + 0.99 * (1 - d) * ct(torch.cat([n, 2 * torch.tanh(at(n))], 1))
         loss = ((critic(torch.cat([o, a], 1)) - y) ** 2).mean()
+        if algo == "td3":
+            loss = loss + ((critic2(torch.cat([o, a], 1)) - y) ** 2).mean()
         oc.zero_grad(); loss.backward(); oc.step()
         if i % 2 == 1:
             al = -critic(torch.cat([o, 2 * torch.tanh(actor(o))], 1)).mean()
             oa.zero_grad(); al.backward(); oa.step()
             with torch.no_grad():
-                for net, tgt in ((actor, at), (critic, ct)):
+                for net, tgt in ((actor, at), (critic, ct)) + (((critic2, ct2),) if algo == "td3" else ()):
                     for p, tp in zip(net.parameters(), tgt.parameters()):
                         tp.mul_(0.995).add_(0.005 * p)
 
@@ -118,6 +137,7 @@ def eager(torch, reps=200):
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--algo", choices=("ddpg", "td3"), default="ddpg")
     ap.add_argument("--iters", type=int, default=2000)
     ap.add_argument("--out", default=None)
     ap.add_argument("--trace-dir", default=None, help="write the profiled run's Chrome trace here")
@@ -126,10 +146,12 @@ def main():
     if not torch.cuda.is_available():
         sys.exit("ddpg_bench needs a GPU")
     res = {**card()}
-    res["n4096"] = timed(torch, 4096, args.iters)
-    res["n1"] = timed(torch, 1, args.iters * 5)
-    res["profile_n4096"] = profiled(torch, 200, args.trace_dir)
-    res.update(eager(torch))
+    if args.algo != "ddpg":
+        res["algo"] = args.algo
+    res["n4096"] = timed(torch, 4096, args.iters, args.algo)
+    res["n1"] = timed(torch, 1, args.iters * 5, args.algo)
+    res["profile_n4096"] = profiled(torch, 200, args.trace_dir, args.algo)
+    res.update(eager(torch, algo=args.algo))
     line = json.dumps(res)
     print(line)
     if args.out:
