@@ -1,7 +1,8 @@
 """Float64 NumPy restatement of DDPG as include/cleanrl_ddpg.h pins it: the nets, both losses and their gradients,
-Adam, Polyak averaging and the run loop. The run loop takes its random draws from the oracle's Philox (olib.philox) and
+Adam, Polyak averaging and the run loop. The run loop takes its random draws from the oracle's Philox (olib.philox; the
+per-env acting draws from philox_draw_many, a NumPy Philox that tests/test_ddpg.py pins to olib.philox bit for bit) and
 its env steps and resets from the oracle's Float32 Pendulum (olib.env_step_raw, olib.reset_uniforms, olib.env_reset_raw),
-so it needs nothing but those three stateless helpers."""
+so it needs nothing but those stateless helpers."""
 import numpy as np
 
 H = 64
@@ -132,6 +133,25 @@ def philox_draw(olib, seed, word, counter, stream):
     return olib.philox([word, counter & 0xFFFFFFFF, counter >> 32, stream], [seed & 0xFFFFFFFF, seed >> 32]).astype(np.uint64)
 
 
+def philox_draw_many(seed, words, counter, stream):
+    """philox_draw of device_math.cuh (Philox4x32-10, ctr = (word, counter lo, counter hi, stream), key = seed) for every
+    entry of `words` at once: [len(words), 4] uint64, bit for bit philox_draw's. Every product of two 32-bit words fits
+    in uint64, so the rounds need no wider type."""
+    m32 = np.uint64(0xFFFFFFFF)
+    c0 = np.asarray(words, np.uint64).ravel()
+    n = len(c0)
+    c1 = np.full(n, counter & 0xFFFFFFFF, np.uint64)
+    c2 = np.full(n, counter >> 32, np.uint64)
+    c3 = np.full(n, stream, np.uint64)
+    k0, k1 = seed & 0xFFFFFFFF, seed >> 32
+    for _ in range(10):
+        p0 = np.uint64(0xD2511F53) * c0
+        p1 = np.uint64(0xCD9E8D57) * c2
+        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ np.uint64(k0), p1 & m32, (p0 >> np.uint64(32)) ^ c3 ^ np.uint64(k1), p0 & m32
+        k0, k1 = (k0 + 0x9E3779B9) & 0xFFFFFFFF, (k1 + 0xBB67AE85) & 0xFFFFFFFF
+    return np.stack([c0, c1, c2, c3], axis=1)
+
+
 def batch_indices(olib, seed, learn_step, size, B):
     keys = np.concatenate([philox_draw(olib, seed, 0, learn_step, STREAM_BATCH), philox_draw(olib, seed, 0x80000000, learn_step, STREAM_BATCH)])
     return perm_index(np.arange(B), size, keys)
@@ -167,7 +187,7 @@ class RefDDPG:
     def _actions(self, obs):
         cfg, N = self.cfg, self.cfg.num_envs
         gs = self.it * N
-        r = np.stack([philox_draw(self.o, cfg.seed, n, self.it, STREAM_ACT) for n in range(N)])
+        r = philox_draw_many(cfg.seed, np.arange(N), self.it, STREAM_ACT)
         if gs <= cfg.learning_starts:
             u = (r[:, 0] >> 8).astype(np.float32) * np.float32(1.0 / 16777216.0)
             return (np.float32(4.0) * u - np.float32(2.0)).astype(np.float32)

@@ -8,10 +8,10 @@ import ddpg_reference as R
 STREAM_SMOOTH = 7
 
 
-def smoothing_normals(olib, seed, learn_step, B):
+def smoothing_normals(seed, learn_step, B):
     """z_b of sample b = 0..B-1 at learning step `learn_step`: Box-Muller of the first two words of
     Philox(seed, word = b, counter = learn_step, stream 7), as the acting kernel forms its noise"""
-    r = np.stack([R.philox_draw(olib, seed, b, learn_step, STREAM_SMOOTH) for b in range(B)])
+    r = R.philox_draw_many(seed, np.arange(B), learn_step, STREAM_SMOOTH)
     u1 = ((r[:, 0] >> 8) + 1).astype(np.float64) / 16777216.0
     u2 = (r[:, 1] >> 8).astype(np.float64) / 16777216.0
     return np.sqrt(-2.0 * np.log(u1)) * np.cos(2.0 * np.pi * u2)
@@ -56,7 +56,7 @@ class RefTD3(R.RefDDPG):
     def learn(self):
         cfg = self.cfg
         idx = R.batch_indices(self.o, cfg.seed, self.learn_steps, self.size, cfg.batch_size)
-        z = smoothing_normals(self.o, cfg.seed, self.learn_steps, cfg.batch_size)
+        z = smoothing_normals(cfg.seed, self.learn_steps, cfg.batch_size)
         self.critic_loss, self.qf2_loss, g1, g2 = twin_critic_loss_grad(
             self.actor_tgt, self.critic, self.qf2, self.critic_tgt, self.qf2_tgt, self.b_obs[idx], self.b_act[idx],
             self.b_rew[idx], self.b_next[idx], self.b_term[idx], cfg.gamma, z, cfg.policy_noise, cfg.noise_clip)

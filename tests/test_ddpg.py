@@ -103,6 +103,22 @@ def test_reference_batch_is_a_sample_without_replacement_matching_the_oracle_per
     assert len(set(idx.tolist())) == 256 and idx.max() < 1000
 
 
+def test_numpy_philox_matches_the_oracle_bit_for_bit(olib):
+    """philox_draw_many, the reference's vectorised Philox4x32-10 for the acting and smoothing draws, against olib.philox:
+    random and extreme words, counters below, at and above 2^32, seeds below, at and above 2^32, and every stream the
+    DDPG kernels use"""
+    rng = np.random.default_rng(12)
+    words = np.concatenate([[0, 1, 0x7FFFFFFF, 0x80000000, 0xFFFFFFFF], rng.integers(0, 1 << 32, 27)]).astype(np.uint64)
+    seeds = [0, 1, 0xFFFFFFFF, 1 << 32, 0x5EED_0001_0002, (1 << 64) - 1] + [int(x) for x in rng.integers(1 << 32, 1 << 63, 2)]
+    counters = [0, 9, 0xFFFFFFFF, 1 << 32, (1 << 40) + 3, (1 << 64) - 1] + [int(x) for x in rng.integers(1 << 32, 1 << 63, 2)]
+    for seed in seeds:
+        for counter in counters:
+            for stream in (R.STREAM_ACT, R.STREAM_BATCH, 7):
+                got = R.philox_draw_many(seed, words, counter, stream)
+                want = np.stack([R.philox_draw(olib, seed, int(w), counter, stream) for w in words])
+                assert got.dtype == np.uint64 and np.array_equal(got, want), (seed, counter, stream)
+
+
 def test_reference_run_loop_counts_and_warmup_ring(olib, abi):
     cfg = abi.make_ddpg_config(num_envs=3, buffer_size=40, learning_starts=30, batch_size=8, train_freq=2, policy_frequency=3,
                                max_episode_steps=7)

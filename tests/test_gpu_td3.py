@@ -49,10 +49,10 @@ BATCHES = [1, 15, 16, 17, 31, 32, 33, 100, 255, 256]
 @pytest.mark.parametrize("kind", KINDS)
 def test_td3_critic_loss_raw_matches_float64(crl, olib, torch_cuda, kind, B):
     """both gradients per parameter array at rtol 1e-4 with atol 2e-6 max|g| (DDPG's tolerance), the losses at rtol 1e-6;
-    the smoothing noise is drawn inside the kernel and by the reference from olib.philox on stream 7"""
+    the smoothing noise is drawn inside the kernel and by the reference from Philox stream 7 (philox_draw_many)"""
     d = td3_batch(kind, B, 9 * B + KINDS.index(kind))
     g1, g2, l1, l2 = gpu_twin(crl, torch_cuda, d)
-    z = T.smoothing_normals(olib, SEED, d["learn_step"], B)
+    z = T.smoothing_normals(SEED, d["learn_step"], B)
     r1, r2, rg1, rg2 = T.twin_critic_loss_grad(d["at"], d["q1"], d["q2"], d["q1t"], d["q2t"], d["obs"], d["act"], d["rew"],
                                                d["nobs"], d["term"], d["gamma"], z, d["pn"], d["nc"])
     np.testing.assert_allclose([l1, l2], [r1, r2], rtol=1e-6)

@@ -127,19 +127,19 @@ def test_reference_twin_critic_matches_torch_autograd_of_cleanrl(kind, B):
 
 def test_smoothing_draw_is_philox_stream_7_keyed_by_batch_position_and_learning_step(olib):
     seed, step, B = 0x1234_5678_9ABC, (1 << 32) + 5, 40
-    z = T.smoothing_normals(olib, seed, step, B)
+    z = T.smoothing_normals(seed, step, B)
     for b in (0, 1, B - 1):
         r = olib.philox([b, step & 0xFFFFFFFF, step >> 32, 7], [seed & 0xFFFFFFFF, seed >> 32])
         u1 = ((int(r[0]) >> 8) + 1) / 16777216.0
         u2 = (int(r[1]) >> 8) / 16777216.0
         assert z[b] == np.sqrt(-2.0 * np.log(u1)) * np.cos(2.0 * np.pi * u2)
     # the draw depends on the step (counter) and on the seed, and differs from DDPG's acting stream 5
-    assert not np.array_equal(z, T.smoothing_normals(olib, seed, step + 1, B))
-    assert not np.array_equal(z, T.smoothing_normals(olib, seed + 1, step, B))
+    assert not np.array_equal(z, T.smoothing_normals(seed, step + 1, B))
+    assert not np.array_equal(z, T.smoothing_normals(seed + 1, step, B))
     r5 = olib.philox([0, step & 0xFFFFFFFF, step >> 32, 5], [seed & 0xFFFFFFFF, seed >> 32])
     r7 = olib.philox([0, step & 0xFFFFFFFF, step >> 32, 7], [seed & 0xFFFFFFFF, seed >> 32])
     assert not np.array_equal(r5, r7)
-    z = T.smoothing_normals(olib, 3, 0, 4000)
+    z = T.smoothing_normals(3, 0, 4000)
     assert abs(z.mean()) < 0.1 and abs(z.std() - 1.0) < 0.1
 
 
