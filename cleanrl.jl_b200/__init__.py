@@ -9,7 +9,8 @@ nothing — the library is dlopen'ed on first use and there is no CPU fallback.
 from . import _abi  # noqa: F401
 from .config import PPOConfig, argparse_struct  # noqa: F401
 
-__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "DDPGConfig", "TD3Config", "argparse_struct", "ppo", "a2c", "dqn", "ddpg", "td3", "PPOHandle", "Networks", "Logger",
+__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "DDPGConfig", "TD3Config", "SACConfig", "argparse_struct", "ppo", "a2c", "dqn", "ddpg", "td3", "sac",
+           "PPOHandle", "Networks", "Logger",
            "ConfigParser"]
 
 
@@ -43,7 +44,16 @@ def td3(*args, **kwargs):
     return _td3(*args, **kwargs)
 
 
+def sac(*args, **kwargs):
+    """Vectorised SAC on Pendulum (pinned to include/cleanrl_sac.h; the reference has no SAC); see sac_algo.py"""
+    from .sac_algo import sac as _sac
+    return _sac(*args, **kwargs)
+
+
 def __getattr__(name):
+    if name == "SACConfig":
+        from .sac_algo import SACConfig
+        return SACConfig
     if name == "TD3Config":
         from .td3_algo import TD3Config
         return TD3Config

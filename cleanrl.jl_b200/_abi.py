@@ -136,3 +136,33 @@ def make_td3_config(num_envs=1, buffer_size=1_000_000, learning_starts=25_000, b
     return crl_td3_config(C.sizeof(crl_td3_config), num_envs, buffer_size, learning_starts, batch_size, train_freq,
                           policy_frequency, max_episode_steps, device, 0, gamma, tau, lr, exploration_noise, seed,
                           policy_noise, noise_clip)
+
+
+# ---- SAC (include/cleanrl_sac.h) -----------------------------------------------------------------------------
+CRL_SAC_ACTOR_PARAMS = 4546
+
+
+class crl_sac_config(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_int32), ("num_envs", C.c_int32), ("buffer_size", C.c_int32), ("learning_starts", C.c_int32),
+        ("batch_size", C.c_int32), ("train_freq", C.c_int32), ("policy_frequency", C.c_int32),
+        ("target_network_frequency", C.c_int32), ("max_episode_steps", C.c_int32), ("device", C.c_int32),
+        ("autotune", C.c_int32), ("_pad", C.c_int32),
+        ("gamma", C.c_double), ("tau", C.c_double), ("policy_lr", C.c_double), ("q_lr", C.c_double), ("alpha", C.c_double),
+        ("seed", C.c_uint64),
+    ]
+
+
+class crl_sac_stats(C.Structure):
+    _fields_ = [("qf1_loss", C.c_double), ("qf2_loss", C.c_double), ("actor_loss", C.c_double), ("alpha_loss", C.c_double),
+                ("alpha", C.c_double), ("sum_return", C.c_double), ("sum_length", C.c_double), ("episodes", C.c_int64),
+                ("learn_steps", C.c_int64), ("actor_steps", C.c_int64), ("iterations", C.c_int64), ("kernel_launches", C.c_int64)]
+
+
+def make_sac_config(num_envs=1, buffer_size=1_000_000, learning_starts=5_000, batch_size=256, train_freq=1, policy_frequency=2,
+                    target_network_frequency=1, max_episode_steps=200, device=0, autotune=1, gamma=0.99, tau=0.005,
+                    policy_lr=3e-4, q_lr=1e-3, alpha=0.2, seed=1):
+    """crl_sac_config with CleanRL's sac_continuous_action.py defaults (PendulumEnv() max_steps = 200)."""
+    return crl_sac_config(C.sizeof(crl_sac_config), num_envs, buffer_size, learning_starts, batch_size, train_freq,
+                          policy_frequency, target_network_frequency, max_episode_steps, device, autotune, 0, gamma, tau,
+                          policy_lr, q_lr, alpha, seed)

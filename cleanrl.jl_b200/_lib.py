@@ -107,6 +107,21 @@ TD3_SIGNATURES = {
     "crl_td3_critic_loss_raw": (C.c_int, [V] * 5 + [I32] + [V] * 5 + [F64, F64, F64, U64, U64] + [V] * 5),
 }
 
+# every symbol include/cleanrl_sac.h declares (the SAC handle and its raw kernels)
+SAC_SIGNATURES = {
+    "crl_sac_create": (C.c_int, [C.POINTER(_abi.crl_sac_config), C.POINTER(V)]),
+    "crl_sac_destroy": (C.c_int, [V]),
+    "crl_sac_set_params": (C.c_int, [V, V, I32, V, I32, V, I32]),
+    "crl_sac_get_params": (C.c_int, [V] * 7),
+    "crl_sac_get_adam_state": (C.c_int, [V] * 9),
+    "crl_sac_reset": (C.c_int, [V]),
+    "crl_sac_run": (C.c_int, [V, I64, V]),
+    "crl_sac_read_buffer": (C.c_int, [V] * 8),
+    "crl_sac_forward_raw": (C.c_int, [V] * 7 + [I64, V]),
+    "crl_sac_critic_loss_raw": (C.c_int, [V] * 5 + [I32] + [V] * 5 + [F64, F64, U64, U64] + [V] * 5),
+    "crl_sac_actor_loss_raw": (C.c_int, [V, V, V, I32, V, F64, U64, U64, V, V, V, V]),
+}
+
 
 def load():
     """dlopen the CUDA library and bind every entry point. Raises if it is not built."""
@@ -117,7 +132,8 @@ def load():
         raise CleanRLCudaError(-2, "%s is not built (run `python cleanrl.jl_b200/build.py` or "
                                    "__graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = C.CDLL(LIB_PATH, mode=C.RTLD_GLOBAL)
-    for name, (res, args) in list(SIGNATURES.items()) + list(DDPG_SIGNATURES.items()) + list(TD3_SIGNATURES.items()):
+    for name, (res, args) in list(SIGNATURES.items()) + list(DDPG_SIGNATURES.items()) + list(TD3_SIGNATURES.items()) + \
+            list(SAC_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError here = header/library mismatch
         fn.restype = res
         fn.argtypes = args

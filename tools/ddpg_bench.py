@@ -1,4 +1,4 @@
-"""Time crl_ddpg_run (or, with --algo td3, crl_td3_run) on one GPU and print one JSON line.
+"""Time crl_ddpg_run (or, with --algo td3 / sac, crl_td3_run / crl_sac_run) on one GPU and print one JSON line.
 
 Workload: 4,096 Pendulum envs, a 1,048,576-transition ring, batch 256, a learning step every iteration,
 policy_frequency 2, learning_starts 10,000; and the same with num_envs 1 (one learning step per env step, CleanRL's
@@ -12,7 +12,10 @@ update-to-data ratio). Reported:
 TD3 runs the same workload with CleanRL's smoothing noise (0.2, clip 0.5); its learning step is the twin-critic pair
 every step and the actor pair + two Polyak launches on every second step. The kernel filter counts the reused ddpg_*
 kernels as well as the td3_* ones.
-Usage: python tools/ddpg_bench.py [--algo {ddpg,td3}] [--iters 2000] [--out path.json]"""
+SAC runs the same workload with CleanRL's SAC settings (policy_lr 3e-4, q_lr 1e-3, autotune): its learning step is the
+twin-critic pair every step, and on every second step two actor iterations (actor pair + temperature pair each), with
+one Polyak launch for both critics every step. The kernel filter counts ddpg_*, td3_* and sac_* kernels.
+Usage: python tools/ddpg_bench.py [--algo {ddpg,td3,sac}] [--iters 2000] [--out path.json]"""
 import argparse
 import json
 import os
@@ -33,7 +36,12 @@ def card():
 def make(num_envs, algo="ddpg"):
     from cleanrl_jl_b200 import _abi
     kw = dict(num_envs=num_envs, buffer_size=1 << 20, learning_starts=10_000, batch_size=256, train_freq=1, policy_frequency=2, seed=1)
-    if algo == "td3":
+    if algo == "sac":
+        from cleanrl_jl_b200.sac_algo import SACHandle, init_sac_params
+        kw.update(policy_lr=3e-4, q_lr=1e-3, target_network_frequency=1, autotune=1)
+        h = SACHandle(_abi.make_sac_config(**kw))
+        h.set_params(*init_sac_params(1))
+    elif algo == "td3":
         from cleanrl_jl_b200.td3_algo import TD3Handle, init_td3_params
         h = TD3Handle(_abi.make_td3_config(**kw))
         h.set_params(*init_td3_params(1))
@@ -73,7 +81,7 @@ def profiled(torch, iters, out_dir, algo="ddpg"):
     h.close()
     per = {}
     for e in prof.key_averages():
-        if "ddpg" in e.key or "td3" in e.key:
+        if any(k in e.key for k in ("ddpg", "td3", "sac")):
             k = e.key.replace("void ", "").replace("(anonymous namespace)::", "").split("(")[0]
             per[k] = per.get(k, 0.0) + e.device_time_total
     act = sum(v for k, v in per.items() if "act_kernel" in k)
@@ -83,6 +91,59 @@ def profiled(torch, iters, out_dir, algo="ddpg"):
         prof.export_chrome_trace(os.path.join(out_dir, "%s_trace.json" % algo))
     return {"us_per_acting_launch": act / iters, "us_per_learning_step": lrn / max(learn, 1),
             "kernel_us_total": {k: round(v, 1) for k, v in per.items()}}
+
+
+def eager_sac_step(torch, dev):
+    """CleanRL's sac_continuous_action.py learning step in PyTorch eager (two actor and temperature iterations on every
+    second step); returns step(i)"""
+    import copy
+    nn = torch.nn
+    mlp = lambda i, o: nn.Sequential(nn.Linear(i, 64), nn.ReLU(), nn.Linear(64, 64), nn.ReLU(), nn.Linear(64, o)).to(dev)
+    actor, qf1, qf2 = mlp(3, 2), mlp(4, 1), mlp(4, 1)
+    qt1, qt2 = copy.deepcopy(qf1), copy.deepcopy(qf2)
+    log_alpha = torch.zeros(1, requires_grad=True, device=dev)
+    oq = torch.optim.Adam(list(qf1.parameters()) + list(qf2.parameters()), lr=1e-3)
+    oa, oal = torch.optim.Adam(actor.parameters(), lr=3e-4), torch.optim.Adam([log_alpha], lr=1e-3)
+    C, B = 1 << 20, 256
+    obs, nobs = torch.randn(C, 3, device=dev), torch.randn(C, 3, device=dev)
+    act, rew, term = torch.rand(C, 1, device=dev) * 4 - 2, torch.randn(C, 1, device=dev), torch.zeros(C, 1, device=dev)
+
+    def get_action(x):
+        mean, log_std = actor(x).chunk(2, dim=1)
+        log_std = -5 + 3.5 * (torch.tanh(log_std) + 1)
+        std = log_std.exp()
+        x_t = mean + std * torch.randn_like(mean)
+        y_t = torch.tanh(x_t)
+        lp = torch.distributions.Normal(mean, std).log_prob(x_t) - torch.log(2 * (1 - y_t.pow(2)) + 1e-6)
+        return 2 * y_t, lp
+
+    def step(i):
+        idx = torch.randperm(C, device=dev)[:B]
+        o, a, r, n, d = obs[idx], act[idx], rew[idx], nobs[idx], term[idx]
+        alpha = log_alpha.exp().item()
+        with torch.no_grad():
+            na, nlp = get_action(n)
+            xn = torch.cat([n, na], 1)
+            y = r + 0.99 * (1 - d) * (torch.min(qt1(xn), qt2(xn)) - alpha * nlp)
+        x = torch.cat([o, a], 1)
+        loss = ((qf1(x) - y) ** 2).mean() + ((qf2(x) - y) ** 2).mean()
+        oq.zero_grad(); loss.backward(); oq.step()
+        if i % 2 == 1:
+            for _ in range(2):
+                pi, lp = get_action(o)
+                xp = torch.cat([o, pi], 1)
+                al = (alpha * lp - torch.min(qf1(xp), qf2(xp))).mean()
+                oa.zero_grad(); al.backward(); oa.step()
+                with torch.no_grad():
+                    _, lp = get_action(o)
+                tl = (-log_alpha.exp() * (lp - 1.0)).mean()
+                oal.zero_grad(); tl.backward(); oal.step()
+                alpha = log_alpha.exp().item()
+        with torch.no_grad():
+            for net, tgt in ((qf1, qt1), (qf2, qt2)):
+                for p, tp in zip(net.parameters(), tgt.parameters()):
+                    tp.mul_(0.995).add_(0.005 * p)
+    return step
 
 
 def eager(torch, reps=200, algo="ddpg"):
@@ -125,6 +186,8 @@ def eager(torch, reps=200, algo="ddpg"):
                     for p, tp in zip(net.parameters(), tgt.parameters()):
                         tp.mul_(0.995).add_(0.005 * p)
 
+    if algo == "sac":
+        step = eager_sac_step(torch, dev)
     for i in range(20):
         step(i)
     torch.cuda.synchronize()
@@ -137,7 +200,7 @@ def eager(torch, reps=200, algo="ddpg"):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--algo", choices=("ddpg", "td3"), default="ddpg")
+    ap.add_argument("--algo", choices=("ddpg", "td3", "sac"), default="ddpg")
     ap.add_argument("--iters", type=int, default=2000)
     ap.add_argument("--out", default=None)
     ap.add_argument("--trace-dir", default=None, help="write the profiled run's Chrome trace here")
