@@ -9,7 +9,8 @@ nothing — the library is dlopen'ed on first use and there is no CPU fallback.
 from . import _abi  # noqa: F401
 from .config import PPOConfig, argparse_struct  # noqa: F401
 
-__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "DDPGConfig", "TD3Config", "SACConfig", "argparse_struct", "ppo", "a2c", "dqn", "ddpg", "td3", "sac",
+__all__ = ["PPOConfig", "A2CConfig", "DQNConfig", "DDPGConfig", "TD3Config", "SACConfig", "C51Config", "argparse_struct", "ppo", "a2c", "dqn", "ddpg", "td3",
+           "sac", "c51",
            "PPOHandle", "Networks", "Logger",
            "ConfigParser"]
 
@@ -50,7 +51,16 @@ def sac(*args, **kwargs):
     return _sac(*args, **kwargs)
 
 
+def c51(*args, **kwargs):
+    """Vectorised C51 on CartPole (pinned to include/cleanrl_c51.h; the reference has no C51); see c51_algo.py"""
+    from .c51_algo import c51 as _c51
+    return _c51(*args, **kwargs)
+
+
 def __getattr__(name):
+    if name == "C51Config":
+        from .c51_algo import C51Config
+        return C51Config
     if name == "SACConfig":
         from .sac_algo import SACConfig
         return SACConfig

@@ -166,3 +166,34 @@ def make_sac_config(num_envs=1, buffer_size=1_000_000, learning_starts=5_000, ba
     return crl_sac_config(C.sizeof(crl_sac_config), num_envs, buffer_size, learning_starts, batch_size, train_freq,
                           policy_frequency, target_network_frequency, max_episode_steps, device, autotune, 0, gamma, tau,
                           policy_lr, q_lr, alpha, seed)
+
+
+# ---- C51 (include/cleanrl_c51.h) -----------------------------------------------------------------------------
+CRL_C51_ATOMS = 101
+CRL_C51_PARAMS = 27934
+
+
+class crl_c51_config(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_int32), ("num_envs", C.c_int32), ("buffer_size", C.c_int32), ("learning_starts", C.c_int32),
+        ("batch_size", C.c_int32), ("train_frequency", C.c_int32), ("target_network_frequency", C.c_int32),
+        ("max_episode_steps", C.c_int32), ("device", C.c_int32), ("_pad", C.c_int32),
+        ("lr", C.c_double), ("gamma", C.c_double), ("start_e", C.c_double), ("end_e", C.c_double),
+        ("epsilon_duration", C.c_double), ("v_min", C.c_double), ("v_max", C.c_double), ("seed", C.c_uint64),
+    ]
+
+
+class crl_c51_stats(C.Structure):
+    _fields_ = [("loss", C.c_double), ("q_values", C.c_double), ("sum_return", C.c_double), ("sum_length", C.c_double),
+                ("epsilon", C.c_double), ("episodes", C.c_int64), ("learn_steps", C.c_int64), ("target_copies", C.c_int64),
+                ("iterations", C.c_int64), ("kernel_launches", C.c_int64)]
+
+
+def make_c51_config(num_envs=1, buffer_size=10_000, learning_starts=10_000, batch_size=128, train_frequency=10,
+                    target_network_frequency=500, max_episode_steps=500, device=0, lr=2.5e-4, gamma=0.99, start_e=1.0,
+                    end_e=0.05, epsilon_duration=250_000.0, v_min=-100.0, v_max=100.0, seed=1):
+    """crl_c51_config with CleanRL's c51.py defaults (epsilon_duration = exploration_fraction 0.5 x total_timesteps
+    500,000; CartPole-v1's 500-step limit)."""
+    return crl_c51_config(C.sizeof(crl_c51_config), num_envs, buffer_size, learning_starts, batch_size, train_frequency,
+                          target_network_frequency, max_episode_steps, device, 0, lr, gamma, start_e, end_e,
+                          epsilon_duration, v_min, v_max, seed)

@@ -122,6 +122,20 @@ SAC_SIGNATURES = {
     "crl_sac_actor_loss_raw": (C.c_int, [V, V, V, I32, V, F64, U64, U64, V, V, V, V]),
 }
 
+# every symbol include/cleanrl_c51.h declares (the C51 handle and its raw kernels)
+C51_SIGNATURES = {
+    "crl_c51_create": (C.c_int, [C.POINTER(_abi.crl_c51_config), C.POINTER(V)]),
+    "crl_c51_destroy": (C.c_int, [V]),
+    "crl_c51_set_params": (C.c_int, [V, V, I32]),
+    "crl_c51_get_params": (C.c_int, [V, V, V, I32]),
+    "crl_c51_get_adam_state": (C.c_int, [V, V, V, V]),
+    "crl_c51_reset": (C.c_int, [V]),
+    "crl_c51_run": (C.c_int, [V, I64, V]),
+    "crl_c51_read_buffer": (C.c_int, [V] * 8),
+    "crl_c51_forward_raw": (C.c_int, [V, V, F64, F64, V, V, V, I64, V]),
+    "crl_c51_loss_raw": (C.c_int, [V, V, I32] + [V] * 5 + [F64, F64, F64, V, V, V, V]),
+}
+
 
 def load():
     """dlopen the CUDA library and bind every entry point. Raises if it is not built."""
@@ -133,7 +147,7 @@ def load():
                                    "__graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = C.CDLL(LIB_PATH, mode=C.RTLD_GLOBAL)
     for name, (res, args) in list(SIGNATURES.items()) + list(DDPG_SIGNATURES.items()) + list(TD3_SIGNATURES.items()) + \
-            list(SAC_SIGNATURES.items()):
+            list(SAC_SIGNATURES.items()) + list(C51_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError here = header/library mismatch
         fn.restype = res
         fn.argtypes = args

@@ -23,7 +23,7 @@ def needs_build():
     if not os.path.exists(OUT):
         return True
     t = os.path.getmtime(OUT)
-    headers = ("cleanrl_cuda.h", "cleanrl_ddpg.h", "cleanrl_td3.h", "cleanrl_sac.h")
+    headers = ("cleanrl_cuda.h", "cleanrl_ddpg.h", "cleanrl_td3.h", "cleanrl_sac.h", "cleanrl_c51.h")
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", h) for h in headers]
     return any(os.path.getmtime(d) > t for d in deps)
 

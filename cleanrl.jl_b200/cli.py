@@ -1,4 +1,4 @@
-"""Runner: `python -m cleanrl_jl_b200 {ppo,a2c,dqn,ddpg,td3,sac} [--field value ...]`.
+"""Runner: `python -m cleanrl_jl_b200 {ppo,a2c,dqn,ddpg,td3,sac,c51} [--field value ...]`.
 
 The reference leaves this wiring as a TODO ("Make individual file runners e.g experiments/run_ppo.(jl/sh)", README.md:24):
 `ConfigParser.argparse_struct` exists (config_parser.jl:18-40) but nothing calls it. Here every field of the algorithm's
@@ -37,21 +37,30 @@ def _sac_configs():
     return {"sac": SACConfig}
 
 
+def _c51_configs():
+    """C51 on CartPole (include/cleanrl_c51.h): one GPU, not in the reference, on a usage line of its own"""
+    from .c51_algo import C51Config
+    return {"c51": C51Config}
+
+
 def main(argv=None):
     argv = list(sys.argv[1:] if argv is None else argv)
     algos = _configs()
     single = _single_gpu_configs()
     ext = _extension_configs()
     sac_ = _sac_configs()
-    if not argv or argv[0] in ("-h", "--help") or argv[0] not in {**algos, **single, **ext, **sac_}:
+    c51_ = _c51_configs()
+    if not argv or argv[0] in ("-h", "--help") or argv[0] not in {**algos, **single, **ext, **sac_, **c51_}:
         sys.stderr.write("usage: python -m cleanrl_jl_b200 {%s} [--<config field> <value> ...]\n"
                          "       python -m cleanrl_jl_b200 {%s} [--<config field> <value> ...]   (one GPU)\n"
                          "       python -m cleanrl_jl_b200 {%s} [--<config field> <value> ...]   (one GPU, not in the reference)\n"
                          "       python -m cleanrl_jl_b200 {%s} [--<config field> <value> ...]   (one GPU, not in the reference)\n"
+                         "       python -m cleanrl_jl_b200 {%s} [--<config field> <value> ...]   (one GPU, not in the reference)\n"
                          "       (every field of the algorithm's config struct is an option; --help after the algorithm lists them)\n"
-                         % (",".join(sorted(algos)), ",".join(sorted(single)), ",".join(sorted(ext)), ",".join(sorted(sac_))))
+                         % (",".join(sorted(algos)), ",".join(sorted(single)), ",".join(sorted(ext)), ",".join(sorted(sac_)),
+                            ",".join(sorted(c51_))))
         return 2
-    algos = {**algos, **single, **ext, **sac_}
+    algos = {**algos, **single, **ext, **sac_, **c51_}
     from .config import argparse_struct
     algo = argv[0]
     config = argparse_struct(algos[algo](), argv[1:])
@@ -64,8 +73,8 @@ def main(argv=None):
         torch.cuda.set_device(local_rank)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     try:
-        from . import a2c, ddpg, dqn, ppo, sac, td3
-        res = {"ppo": ppo, "a2c": a2c, "dqn": dqn, "ddpg": ddpg, "td3": td3, "sac": sac}[algo](config)
+        from . import a2c, c51, ddpg, dqn, ppo, sac, td3
+        res = {"ppo": ppo, "a2c": a2c, "dqn": dqn, "ddpg": ddpg, "td3": td3, "sac": sac, "c51": c51}[algo](config)
     finally:
         if dist is not None:
             dist.destroy_process_group()
